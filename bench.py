@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the karma k-mer front end (profile matrix + exact kNN graph).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): contigs/s for (profile + kNN).  Workload at every N is
 BASELINE.json configs[1]: a 50 000-contig synthetic Trinity-like assembly (S1 gene
@@ -24,6 +24,9 @@ after the timed region.  Supplementary blocks (outside every timed region): the 
 counting kernel on the 5120-column shape, a parity sample against the fp64 oracle at N>1, and at N=8 the
 500k (BASELINE configs[2]) and 1M-contig (north_star target) runs.
 One JSON line is printed by rank 0.
+
+--dump-outputs DIR writes what the T0 pass left on the device after its last timed step (dump_outputs below):
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -60,6 +63,8 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="enqueue the pass eagerly instead of replaying a CUDA graph")
     ap.add_argument("--shard-gen", action="store_true", help="each rank synthesises only its own row shard")
     ap.add_argument("--big", default=None, help="comma list of contig counts for the sharded 5+6 / k=15 runs (default at N=8: 500000,1000000; 0: none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (a seeded row sample, at most 64 MB)")
     return ap.parse_args()
 
 
@@ -322,6 +327,33 @@ def timed_plan_loop(torch, dist, plan, steps, world):
     return float(t.item()), checks
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, torch, dist, plan, n_total, lo, rank, world):
+    """Write what a caller of PassPlan.run receives after the last pass: profile.npy (float64 profile rows),
+    knn_idx.npy (neighbour indices, int32 held exactly in float64) and knn_dist.npy (float32 distances).  When all
+    rows exceed DUMP_BYTES, a row sample drawn with a fixed seed is written; rows.npy holds the row numbers.  At N>1
+    every rank contributes its profile rows; rank 0 writes."""
+    per_row = plan.cols * 8 + plan.k * (8 + 4) + 8
+    m = min(n_total, (DUMP_BYTES - 4096) // per_row)          # 4096: room for the four .npy headers
+    rows = np.arange(n_total) if m == n_total else np.sort(np.random.default_rng(0).choice(n_total, m, replace=False))
+    mine = rows[(rows >= lo) & (rows < lo + plan.n)] - lo
+    prof = plan.profile[torch.from_numpy(mine).to(plan.profile.device)].cpu().numpy()
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, prof)
+        prof = np.concatenate(parts)
+    if rank != 0:
+        return
+    sel = torch.from_numpy(rows).to(plan.all_idx.device)       # gathered lists: row r of the assembly is row r here
+    arrays = {"rows": rows.astype(np.float64), "profile": prof,
+              "knn_idx": plan.all_idx[sel].cpu().numpy().astype(np.float64), "knn_dist": plan.all_dist[sel].cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def big_run(torch, dist, eng, a, n_total, rank, world, local, pk):
     """One sharded run of the north-star shape (5120 dense columns, n_neighbors = 15): every rank synthesises its
     own row shard.  Device-resident steps, one host-to-host step, and a parity sample of rank 0's rows against
@@ -501,6 +533,8 @@ def run_ours(a):
     total_ms, checks = timed_plan_loop(torch, dist, plan, a.steps, world)
     if not all(c["ok"] for c in checks + [warm]):
         raise RuntimeError("optimistic validation failed on the synthetic assembly: %r" % (checks[-1],))
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, torch, dist, plan, n_total, lo, rank, world)
     uncertified = checks[-1]["uncertified"]
     value = n_total * a.steps / (total_ms / 1e3)
     d_cols = plan.cols

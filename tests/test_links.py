@@ -43,23 +43,6 @@ def test_oracle_matches_reference_golden(lk_golden):
             assert float(lo.distance_between_subgraphs(adj, t["nodes_a"], t["nodes_b"])).hex() == t["weight"], c["name"]
 
 
-@pytest.mark.skipif(not (lo.reference_available() and ro.reference_available()), reason="/root/reference not present")
-def test_oracle_matches_reference_live(tmp_path):
-    names, classes = ro.synth_eq_classes(70, 600, seed=91, family=5, max_size=6, p_cross=0.3)
-    path = str(tmp_path / "eq.txt")
-    ro.write_eq_file(path, names, classes)
-    graph = ro.reference_graph(path, [">" + x for x in names])
-    nodes = list(graph.nodes())
-    adj = lo.adjacency(nodes, [(a, b, d["weight"]) for a, b, d in graph.edges(data=True)])
-    rng = np.random.default_rng(5)
-    order = [nodes[i] for i in rng.permutation(len(nodes))]
-    lookup = lo.lookup_dict([[order[i:i + 7]] for i in range(0, len(order), 7)])
-    for cutoff in (0, 0.4):
-        assert lo.connections_between_subclusters(adj, lookup, cutoff) == lo.reference_connections(graph, lookup, cutoff)
-    a, b = order[:20], order[10:45]
-    assert float(lo.distance_between_subgraphs(adj, a, b)).hex() == float(graph.calc_distance_between_subgraphs(a, b)).hex()
-
-
 def test_roles_and_argument_errors():
     from karma_b200 import rearrange as rr
     index = {"a": 0, "b": 1, "c": 2, "d": 3}

@@ -30,18 +30,6 @@ def test_oracle_matches_reference_golden(rg_golden):
         assert all(r["adj"][int(k)] == v for k, v in c["adj"].items()), c["name"]
 
 
-@pytest.mark.skipif(not ro.reference_available(), reason="/root/reference not present")
-def test_oracle_matches_reference_live(tmp_path):
-    names, classes = ro.synth_eq_classes(50, 400, seed=77, family=5, max_size=7)
-    path = str(tmp_path / "eq.txt")
-    ro.write_eq_file(path, names, classes)
-    keys = [">" + x for x in names]
-    ref = ro.reference_build(path, keys)
-    r = ro.build(names, classes, keys)
-    assert r["nodes"] == ref["nodes"] and [(a, b, w.hex()) for a, b, w in r["edges"]] == [(a, b, w.hex()) for a, b, w in ref["edges"]]
-    assert all(r["adj"][k] == v for k, v in ref["adj"].items())
-
-
 def test_native_parser_matches_python_parser(tmp_path, rg_golden):
     from karma_b200 import read_graph as rg
     for c in rg_golden:
