@@ -274,7 +274,7 @@ KB_API int64_t kb_knn_fixup(kb_ctx* ctx, int impl, int32_t k,
 KB_API int kb_knn_uncertified_ptr(kb_ctx* ctx, int64_t nq, int64_t nk, int64_t q_row0, int32_t d_cols_padded, int32_t k, int impl, int64_t n_flag,
                            void* d_workspace, const uint32_t** d_count);
 /* Host-only views of the tensor kernel's work schedule (tests, diagnostics): kb_knn_plan_info fills
- * out[0..7] = candidate width k', lists per row, key bands, schedule kind, workers (CTA clusters), pieces,
+ * out[0..7] = candidate width k', lists per row, key bands, schedule kind, workers (CTA pairs), pieces,
  * 1000 x tile visits of the busiest worker, 1000 x the ideal; kb_knn_plan_table the table itself:
  * pieces int32[pieces*8] = {group, slot, t_lo, cnt, shift, i_lo, i_cnt, 0}, piece_start int32[workers+1],
  * slot_count int32[groups]. */
@@ -295,8 +295,7 @@ KB_API int kb_knn_plan_table(int sm_count, int impl, int64_t nq, int64_t nk, int
  *   kb_xchg_push     on `stream` (a side stream ordered after K3): wait until every peer is done with the
  *                    previous pass, copy this rank's shard of every region -- bytes [off + rank*shard_bytes,
  *                    +shard_bytes) -- into every peer's arena (copy engines, three peers at a time, nearest-following
- *                    rank first), then arrive[rank] = epoch there.  KB_XCHG_SM=1 pushes with a kernel instead (SM stores
- *                    over NVLink next to the persistent K4 CTAs; measured slower at 8 ranks)
+ *                    rank first), then arrive[rank] = epoch there
  *   kb_knn(..xchg..) sweeps the local shard first and waits for arrive[r] before the first key row of rank r
  *   kb_xchg_finish   on the context stream after K5: copy this rank's record (rec_words u32 at
  *                    rec_off + rank*rec_words*4) to every peer, raise the results flag everywhere and wait

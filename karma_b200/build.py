@@ -37,9 +37,6 @@ def _stale(target, deps):
 
 def build(force=False, verbose=False):
     os.makedirs(OBJ, exist_ok=True)
-    extra = os.environ.get("KB_NVCC_EXTRA", "").split()      # e.g. -DKB_TC_STATS for experiments
-    if extra:
-        force = True
     nvcc = _nvcc()
     hdrs = [os.path.join(CSRC, h) for h in HEADERS]
     jobs = []
@@ -51,7 +48,7 @@ def build(force=False, verbose=False):
 
     def compile_one(job):
         s, o = job
-        cmd = [nvcc] + NVCC_FLAGS + extra + ["-c", s, "-o", o]
+        cmd = [nvcc] + NVCC_FLAGS + ["-c", s, "-o", o]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (s, r.stdout, r.stderr))

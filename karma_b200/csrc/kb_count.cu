@@ -827,7 +827,6 @@ int launch(kb_ctx* ctx, const uint8_t* d_bases, const int64_t* d_offsets, int64_
         if (n < 8 * resident_warps) lp.batch = 2;
         if (n < 4 * resident_warps) lp.batch = 1;
         if (n < 2 * resident_warps) lp.rows1 = 8;                // few contigs: finer class-1 tickets keep every CTA busy
-        if (const char* e = getenv("KB_K1_FIRST")) { const long v = atol(e); if (v >= 64) lp.first = v; }   // experiments only
         int64_t grid = (int64_t)ctx->sm_count * per_sm;         // persistent: one resident wave
         const int64_t want = (n + WARPS - 1) / WARPS;
         if (grid > want) grid = want;

@@ -135,14 +135,11 @@ void choose_sched(const KbKnnPlan& p, int64_t q_row0, const int* min_bands, bool
     static const int cand[] = {1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 14, 16, 20, 24, 28, 32, 40, 48, 64};
     const int max_slots = KB_KNN_MAX_CAND / p.kp;
     bool have = false;
-    const char* fs = getenv("KB_KNN_SPLITS");                            // experiments only
-    const char* fk = getenv("KB_KNN_SCHED");                             // experiments only: 0 round-robin units, 1 balanced cut
     for (int S : cand) {
         if (S > p.n_tiles || S > max_slots) break;
-        if (fs && atoi(fs) >= 1 && S != std::min<int64_t>(std::min<int64_t>(atoi(fs), p.n_tiles), max_slots)) continue;
         for (int kind = 0; kind < 2; ++kind) {
-            if (fk ? atoi(fk) != kind : (sync_only && kind == 1)) continue;
-            if (!fs && S < min_bands[kind] && S < p.n_tiles && S < max_slots) continue;
+            if (sync_only && kind == 1) continue;
+            if (S < min_bands[kind] && S < p.n_tiles && S < max_slots) continue;
             Sched s;
             build_sched(p, q_row0, S, kind, &s);
             if (s.slots > max_slots) continue;
@@ -174,15 +171,10 @@ int kb_knn_plan(int sm_count, int impl, int64_t nq, int64_t nk, int64_t q_row0, 
         p->piece_cost = std::min(1.5, std::max(0.25, 1.5 * 1088.0 / (double)dp));
         p->shard = (q_row0 > 0 || nq < nk) ? 1 : 0;
         if (impl == KB_KNN_TC) {
-            int64_t cl = p->m_blocks >= 2 ? 2 : 1;
-            if (const char* f = getenv("KB_KNN_CLUSTER")) {         // experiments only: 1, 2 or 4 CTAs share every key tile
-                const int v = atoi(f);
-                if ((v == 1 || v == 2 || v == 4) && p->m_blocks >= v) cl = v;
-            }
-            p->cl = (int)cl;
-            p->groups = (p->m_blocks + cl - 1) / cl;
-            int64_t w = sm_count / cl > 0 ? sm_count / cl : 1;
-            if (cl == 4) w = std::min<int64_t>(w, 32);              // clusters of 4 live inside one GPC: fewer fit
+            // CTA pairs (k4_tc2), also for a lone query block: the second CTA of its pair has no live rows
+            p->cl = 2;
+            p->groups = (p->m_blocks + 1) / 2;
+            int64_t w = sm_count / 2 > 0 ? sm_count / 2 : 1;
             const int64_t visits = p->groups * p->n_tiles;
             if (w > visits) w = visits;
             p->workers = (int)w;
@@ -190,8 +182,7 @@ int kb_knn_plan(int sm_count, int impl, int64_t nq, int64_t nk, int64_t q_row0, 
             // B200: 126 MB of L2.  A key set that fills a good part of it is swept in bands that all workers share
             // (measured in place, i.e. with the L2 cold after K1-K3: 50k x 1088 keys = 109 MB, one band cut into
             // ranges 3.30 ms, three whole bands dealt round-robin 3.13 ms); beyond the L2 only whole bands are dealt.
-            double l2_mb = 120.0;
-            if (const char* f = getenv("KB_KNN_L2_MB")) l2_mb = atof(f);   // experiments only
+            const double l2_mb = 120.0;
             const double key_bytes = (double)nk * dp * 2.0;
             const bool sync_only = key_bytes > l2_mb * 1e6;
             const bool shard = p->shard != 0;                        // arrival order: at least 4 bands

@@ -6,8 +6,8 @@
 #define KB_KNN_K_MAX 60           // largest k served by the candidate kernels; beyond: exact pass over all keys
 #define KB_KNN_MAX_CAND 512       // K5 merges at most this many candidates per row (slots * KP)
 
-// One piece of work of the tensor kernel: query-block group `group` (CL adjacent 128-row blocks, one
-// per CTA of the cluster) against the key tiles tile(i), i in [i_lo, i_lo + i_cnt), of the sweep
+// One piece of work of the tensor kernel: query-block group `group` (2 adjacent 128-row blocks, one
+// per CTA of the pair) against the key tiles tile(i), i in [i_lo, i_lo + i_cnt), of the sweep
 //     tile(i) = (t_lo + ((i + shift) mod cnt)) mod n_tiles
 // (a band of `cnt` key tiles starting at t_lo -- for a query shard it may wrap round the end of the key set --
 // rotated so that the band holding the group's diagonal starts AT the diagonal).  The running top-KP list of
@@ -18,7 +18,7 @@ struct KbPiece {
 
 // Candidate-search plan.
 //  SIMT kernel: grid (m_blocks, slots); slot s covers key tiles [n_tiles*s/slots, n_tiles*(s+1)/slots).
-//  Tensor kernel: a table of pieces per worker (= CTA cluster), built on the host so that every worker
+//  Tensor kernel: a table of pieces per worker (= CTA pair), built on the host so that every worker
 //  gets the same number of tile visits and all workers sweep the same band of key tiles at the same time.
 struct KbKnnPlan {
     int impl;            // KB_KNN_SIMT / KB_KNN_TC, or 0: no candidate kernel (k > KB_KNN_K_MAX: exact pass only)
@@ -28,9 +28,9 @@ struct KbKnnPlan {
     int64_t n_tiles;     // ceil(nk / bn)
     int64_t nq;          // query rows
     int shard;           // the queries are a row shard of the keys (the other shards arrive over NVLink)
-    int cl;              // tensor path: CTAs per cluster sharing one key-tile stream (1, 2 or 4)
+    int cl;              // query blocks per group: 2 on the tensor path (one per CTA of a pair), 1 on SIMT
     int64_t groups;      // ceil(m_blocks / cl)
-    int workers;         // tensor path: clusters launched
+    int workers;         // tensor path: CTA pairs launched
     int slots;           // candidate lists per query row (upper bound; per group see slot_count)
     int bands;           // tensor path: S
     int sched_kind;      // 0: whole units dealt round-robin, 1: every band cut into equal ranges

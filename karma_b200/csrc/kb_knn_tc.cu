@@ -8,31 +8,31 @@
 //                       in TMEM (exact integer Gram while sum c^2 < 2^24)
 //   score_ij = fma(G_ij, -2/l_j, l_i * n_j/l_j^2)   ( = l_i*d2_ij - n_i/l_i )
 //
-// One persistent CTA per SM, 6 warps:
-//   warp 0      TMA producer: 128x64 (A) and 2 x 128x64 (B) fp16 boxes, SWIZZLE_128B,
-//               STAGES-deep mbarrier ring
-//   warp 1      TMEM allocator + single-thread tcgen05.mma issuer
-//               (cta_group::1, kind::f16, M=128 N=256 K=16), accumulators double
-//               buffered in TMEM (2 x 256 columns)
-//   warps 2-5   epilogue: tcgen05.ld 32 lanes x 32 columns, one thread per query
-//               row; running top-KP list per row in shared memory
-// Work = a host-built table of pieces per cluster (kb_knn.cuh: KbPiece): a query-block group against a
-// run of key tiles; each piece writes KP candidates per row into its slot, merged and exactly reranked
-// by K5 (kb_knn.cu).  With a peer-memory exchange the TMA producer (and the epilogue, for the key
-// records) waits for the arrival flag of the rank that owns a key row before touching it, so the sweep
-// starts on the local shard while the other shards are still in flight over NVLink.
+// k4_tc2: persistent CTA pairs (clusters of 2, one CTA per SM), 6 warps per CTA, ONE 2-CTA MMA per pair:
+//   warp 0      TMA producer (both CTAs): the CTA's 128 query rows x 64 (A) and its half of the key tile,
+//               128 rows x 64 (B), fp16 boxes, SWIZZLE_128B, STAGES-deep mbarrier ring (32 KB per stage)
+//   warp 1      TMEM allocator (both CTAs) + single-thread tcgen05.mma issuer in the leader CTA
+//               (cta_group::2, kind::f16, M=256 N=256 K=16), accumulators double buffered in TMEM
+//               (2 x 256 columns per SM)
+//   warps 2-5   epilogue of the CTA's own 128 rows: tcgen05.ld 32 lanes x 32 columns, one thread per
+//               query row; running top-KP list per row in shared memory
+// Work = a host-built table of pieces per CTA pair (kb_knn.cuh: KbPiece): a group of two adjacent 128-row
+// query blocks against a run of key tiles; each piece writes KP candidates per row into its slot, merged and
+// exactly reranked by K5 (kb_knn.cu).  A group whose second block has no live rows (an odd number of query
+// blocks, or a query range of at most 128 rows) still runs as a pair; the idle CTA's rows are never written.
+// With a peer-memory exchange the TMA producer (and the epilogue, for the key records) waits for the arrival
+// flag of the rank that owns a key row before touching it, so the sweep starts on the local shard while the
+// other shards are still in flight over NVLink.
 //
 // Roofline: tensor pipe.  Algorithmic flops = 2 * nq * nk * D.
 #include "kb_knn.cuh"
 #include <cuda.h>
-#include <cstdlib>
 
 namespace {
 
 constexpr int BM = 128, BN = 256, BK = 64;
 constexpr int A_BYTES = BM * BK * 2;          // 16 KB
 constexpr int B_BYTES = BN * BK * 2;          // 32 KB
-constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
 constexpr int NUM_THREADS = 192;
 constexpr uint32_t TMEM_COLS = 512;
 
@@ -43,9 +43,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
     uint32_t ok;
@@ -69,12 +66,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, int tag
     }
 }
 
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int32_t c0, int32_t c1, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-
 // K-major SWIZZLE_128B shared-memory matrix descriptor (sm_100 "version 1"):
 // rows are 128 B apart, 8-row groups 1024 B apart.
 __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
@@ -87,30 +78,6 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
     return d;
 }
 
-// kind::f16 instruction descriptor: D=F32, A=B=F16, K-major both, N=256, M=128
-constexpr uint32_t IDESC = (1u << 4) | (0u << 7) | (0u << 10) | (0u << 15) | (0u << 16) |
-                           ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// multicast variants (cluster of 2 CTAs that share the B tile)
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* map, int32_t c0, int32_t c1, uint32_t bar, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%4, %5}], [%2], %3;"
-        ::"r"(dst), "l"(map), "r"(bar), "h"(mask), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"(mask) : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
@@ -132,10 +99,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-#ifdef KB_TC_STATS
-__device__ unsigned long long g_tc_inserts, g_tc_cold_chunks, g_tc_chunks;
-#endif
-
 struct TcParams {
     int64_t nk, q_row0, nq;
     int slots;                        // candidate lists per query row (stride of cand_*)
@@ -146,7 +109,7 @@ struct TcParams {
     int32_t* cand_idx;
     int32_t* row_thr;                 // per query row: best known KP-th score (ordered-int key), shared by all pieces
     const KbPiece* pieces;
-    const int32_t* piece_start;       // per cluster
+    const int32_t* piece_start;       // per CTA pair
     const uint32_t* arrive;           // peer exchange (nullable): arrive[r] >= *epoch once rank r's shard has landed
     const uint32_t* epoch;
     int64_t rows_per_src;
@@ -192,234 +155,15 @@ __device__ __forceinline__ void wait_row_arrived(const TcParams& p, uint32_t epo
 __device__ __forceinline__ int32_t f2key(float f) { const int32_t i = __float_as_int(f); return i >= 0 ? i : i ^ 0x7fffffff; }
 __device__ __forceinline__ float key2f(int32_t k) { return __int_as_float(k >= 0 ? k : k ^ 0x7fffffff); }
 
-template <int KP, int STAGES>
-struct Smem {
-    static constexpr int OFF_STAGES = 0;
-    static constexpr int OFF_LIST_S = STAGES * STAGE_BYTES;
-    static constexpr int OFF_LIST_I = OFF_LIST_S + KP * BM * 4;
-    static constexpr int OFF_COLMETA = OFF_LIST_I + KP * BM * 4;
-    static constexpr int OFF_BARS = OFF_COLMETA + BN * 8;
-    // full[STAGES], empty[STAGES], tmem_full[2], tmem_empty[2]
-    static constexpr int OFF_TMEM_SLOT = OFF_BARS + (2 * STAGES + 4) * 8;
-    static constexpr int TOTAL = OFF_TMEM_SLOT + 16;
-};
-
-// CL = 1: stand-alone CTAs.  CL = 2: clusters of two CTAs with adjacent query blocks; each
-// loads half of every B tile and TMA-multicasts it to both, which cuts the L2->SM operand
-// traffic per tile from 384 to 256 rows (the v2 profile had the L2 at 73 % of peak).
-template <int KP, int STAGES, int CL>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-k4_tc(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_b, const TcParams p) {
-    using L = Smem<KP, STAGES>;
-    constexpr int B_PART_ROWS = CL == 1 ? 128 : BN / CL;       // rows of the key tile one TMA brings (box of tmap_b)
-    constexpr uint16_t CL_MASK = (uint16_t)((1u << CL) - 1);
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t sbase = smem_u32(smem);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0 && (sbase & 1023u)) {
-        printf("kb_knn_tc: dynamic shared memory is not 1024-byte aligned (0x%x)\n", sbase);
-        __trap();
-    }
-    const uint32_t bar_full = sbase + L::OFF_BARS;
-    const uint32_t bar_empty = bar_full + STAGES * 8;
-    const uint32_t bar_tfull = bar_empty + STAGES * 8;
-    const uint32_t bar_tempty = bar_tfull + 2 * 8;
-    volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + L::OFF_TMEM_SLOT);
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap_b) : "memory");
-        // a stage is free again once the MMAs of EVERY CTA that receives multicast data into
-        // it have retired: each CTA's commit arrives on all CL empty barriers
-        for (int s = 0; s < STAGES; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, CL); }
-        for (int a = 0; a < 2; ++a) { mbar_init(bar_tfull + 8 * a, 1); mbar_init(bar_tempty + 8 * a, 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     ::"r"(smem_u32((const void*)tmem_slot)), "r"(TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    if constexpr (CL > 1) cluster_sync_all();                // peers' barriers are initialised before any remote arrive
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    const int cta_rank = (CL > 1) ? (int)cluster_ctarank() : 0;
-    const int worker = blockIdx.x / CL;
-    const int32_t pc_lo = p.piece_start[worker], pc_hi = p.piece_start[worker + 1];
-    const uint32_t epoch = p.arrive ? *p.epoch : 0u;
-
-    if (warp == 0) {
-        // ================= TMA producer =================
-        if (lane == 0) {
-            int stage = 0; uint32_t phase = 0;
-            uint32_t seen = 0;
-            for (int32_t pi = pc_lo; pi < pc_hi; ++pi) {
-                const KbPiece pc = load_piece(p.pieces + pi);
-                const int32_t arow = (int32_t)(p.q_row0 + ((int64_t)pc.group * CL + cta_rank) * BM);
-                for (int i = pc.i_lo; i < pc.i_lo + pc.i_cnt; ++i) {
-                    const int32_t brow = (int32_t)(piece_tile(pc, i, p.n_tiles) * BN);
-                    if (p.arrive) {
-                        wait_row_arrived(p, epoch, brow, seen, 1);
-                        wait_row_arrived(p, epoch, (int64_t)brow + BN - 1, seen, 1);
-                        asm volatile("fence.proxy.async;" ::: "memory");
-                    }
-                    for (int kb = 0; kb < p.k_blocks; ++kb) {
-                        mbar_wait(bar_empty + 8 * stage, phase ^ 1, 1);
-                        const uint32_t sa = sbase + L::OFF_STAGES + stage * STAGE_BYTES;
-                        const uint32_t fb = bar_full + 8 * stage;
-                        mbar_expect_tx(fb, STAGE_BYTES);
-                        tma_load_2d(sa, &tmap, kb * BK, arow, fb);
-                        if constexpr (CL == 1) {
-                            tma_load_2d(sa + A_BYTES, &tmap_b, kb * BK, brow, fb);
-                            tma_load_2d(sa + A_BYTES + B_BYTES / 2, &tmap_b, kb * BK, brow + 128, fb);
-                        } else {
-                            // my 1/CL of B goes to the same smem offset (and full barrier) of every CTA of the cluster
-                            tma_load_2d_mc(sa + A_BYTES + cta_rank * (B_BYTES / CL), &tmap_b, kb * BK, brow + B_PART_ROWS * cta_rank, fb, CL_MASK);
-                        }
-                        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ================= MMA issuer =================
-        if (lane == 0) {
-            int stage = 0; uint32_t phase = 0;
-            int acc = 0; uint32_t acc_phase = 0;
-            for (int32_t pi = pc_lo; pi < pc_hi; ++pi) {
-                const KbPiece pc = load_piece(p.pieces + pi);
-                for (int i = 0; i < pc.i_cnt; ++i) {
-                    mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1, 2);
-                    tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + (uint32_t)(acc * BN);
-                    for (int kb = 0; kb < p.k_blocks; ++kb) {
-                        mbar_wait(bar_full + 8 * stage, phase, 3);
-                        tc_fence_after();
-                        const uint32_t sa = sbase + L::OFF_STAGES + stage * STAGE_BYTES;
-                        const uint64_t adesc = make_smem_desc(sa);
-                        const uint64_t bdesc = make_smem_desc(sa + A_BYTES);
-#pragma unroll
-                        for (int k = 0; k < BK / 16; ++k) {
-                            // +32 B per K=16 step inside the 128 B swizzle atom (>>4 => +2)
-                            umma_f16(d_tmem, adesc + 2 * k, bdesc + 2 * k, IDESC, (kb | k) != 0);
-                        }
-                        // frees the smem stage (here and in the peer CTA) when these MMAs retire
-                        if constexpr (CL == 1) umma_commit(bar_empty + 8 * stage);
-                        else umma_commit_mc(bar_empty + 8 * stage, CL_MASK);
-                        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                    }
-                    umma_commit(bar_tfull + 8 * acc);                // accumulator ready for the epilogue
-                    if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-                }
-            }
-        }
-    } else {
-        // ================= epilogue: warps 2..5 =================
-        const int quad = warp & 3;                           // TMEM lane quadrant this warp may read
-        const int r = quad * 32 + lane;                      // row of the 128-row tile
-        const int et = threadIdx.x - 64;                     // 0..127
-        KbRowList<KP, BM> list(reinterpret_cast<float*>(smem + L::OFF_LIST_S),
-                               reinterpret_cast<int32_t*>(smem + L::OFF_LIST_I));
-        const float4* cm4 = reinterpret_cast<const float4*>(smem + L::OFF_COLMETA);
-        float2* cm_s = reinterpret_cast<float2*>(smem + L::OFF_COLMETA);
-        int acc = 0; uint32_t acc_phase = 0;
-        uint32_t seen = 0;
-        for (int32_t pi = pc_lo; pi < pc_hi; ++pi) {
-            const KbPiece pc = load_piece(p.pieces + pi);
-            const int64_t q = ((int64_t)pc.group * CL + cta_rank) * BM + r;
-            const bool live = q < p.nq;
-            const float li = live ? (float)p.rowmeta[p.q_row0 + q].key_len : 1.f;
-            list.init(r);
-            float thr = __int_as_float(0x7f800000);          // min(own KP-th best, row_thr): the prune bound
-            for (int i = pc.i_lo; i < pc.i_lo + pc.i_cnt; ++i) {
-                const int64_t n0 = piece_tile(pc, i, p.n_tiles) * BN;
-                // stage this tile's key records (all 128 epilogue threads); refresh the shared bound
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                if (p.arrive) { wait_row_arrived(p, epoch, n0 + et, seen, 5); wait_row_arrived(p, epoch, n0 + et + 128, seen, 5); }
-                cm_s[et] = kb_load_cm(p.rowmeta, n0 + et, p.nk);
-                cm_s[et + 128] = kb_load_cm(p.rowmeta, n0 + et + 128, p.nk);
-                if (live) thr = fminf(thr, key2f(__ldcg(p.row_thr + q)));
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                mbar_wait(bar_tfull + 8 * acc, acc_phase, 4);
-                tc_fence_after();
-                const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN);
-#pragma unroll 1
-                for (int c = 0; c < BN / 32; ++c) {
-                    uint32_t v[32];
-                    tmem_ld32(taddr + c * 32, v);
-                    tmem_ld_wait();
-                    // hot path: branch-free scores + chunk minimum
-                    float sc[32];
-                    float m0 = thr, m1 = thr, m2 = thr, m3 = thr;
-#pragma unroll
-                    for (int x = 0; x < 32; x += 2) {
-                        const float4 cm = cm4[c * 16 + (x >> 1)];
-                        sc[x] = fmaf(__uint_as_float(v[x]), cm.x, li * cm.y);
-                        sc[x + 1] = fmaf(__uint_as_float(v[x + 1]), cm.z, li * cm.w);
-                    }
-#pragma unroll
-                    for (int x = 0; x < 32; x += 4) {
-                        m0 = fminf(m0, sc[x]); m1 = fminf(m1, sc[x + 1]);
-                        m2 = fminf(m2, sc[x + 2]); m3 = fminf(m3, sc[x + 3]);
-                    }
-#ifdef KB_TC_STATS
-                    if (lane == 0) atomicAdd(&g_tc_chunks, 1ull);
-                    if (__any_sync(0xffffffffu, fminf(fminf(m0, m1), fminf(m2, m3)) < thr) && lane == 0) atomicAdd(&g_tc_cold_chunks, 1ull);
-#endif
-                    if (fminf(fminf(m0, m1), fminf(m2, m3)) < thr) {
-                        // cold path: some element of this chunk beats the bound
-#pragma unroll
-                        for (int x = 0; x < 32; ++x) {
-                            if (sc[x] < thr) {
-                                list.insert(r, sc[x], (int32_t)(n0 + c * 32 + x));
-                                thr = fminf(thr, list.bound);
-#ifdef KB_TC_STATS
-                                atomicAdd(&g_tc_inserts, 1ull);
-#endif
-                            }
-                        }
-                    }
-                }
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-                // publish a full list's bound for the other units of these rows
-                if (live && list.bound < __int_as_float(0x7f800000)) atomicMin(p.row_thr + q, f2key(list.bound));
-            }
-            if (live) {
-                const int64_t base = (q * p.slots + pc.slot) * KP;
-#pragma unroll
-                for (int e = 0; e < KP; ++e) {
-                    p.cand_score[base + e] = list.s[e * BM + r];
-                    p.cand_idx[base + e] = list.i[e * BM + r];
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if constexpr (CL > 1) cluster_sync_all();                // no CTA leaves while its peer may still signal it
-    if (warp == 1) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-    }
-}
-
 // =====================================================================================
-// k4_tc2: the same unit/epilogue structure with ONE 2-CTA MMA per CTA pair
-// (tcgen05.mma.cta_group::2, M=256 N=256 K=16).  Each CTA keeps its 128 query rows (A) and
-// HALF of the key tile (128 B rows) in shared memory: 32 KB per stage instead of 48 KB, so
-// the ring is 6 deep, and the tensor core reads B once for both SMs.  The leader CTA (cluster
+// k4_tc2: ONE 2-CTA MMA per CTA pair (tcgen05.mma.cta_group::2, M=256 N=256 K=16).  Each CTA
+// keeps its 128 query rows (A) and HALF of the key tile (128 B rows) in shared memory: 32 KB
+// per stage, so the ring is up to 6 deep, and the tensor core reads B once for both SMs.  The leader CTA (cluster
 // rank 0) issues the MMAs; every TMA of either CTA signals the leader's "full" barrier
 // (.cta_group::2 TMA with the peer-masked barrier address); the leader's commits are multicast
 // to both CTAs' "stage empty" and "accumulator full" barriers; both CTAs' epilogue warps arrive
-// on the leader's "accumulator empty" barrier.  Default for CTA pairs: +0.4 % at 1088 columns, +10 % at 5120
-// (profiles/r01/k4_variants.md); KB_KNN_MMA2=0 selects k4_tc<.,.,2> instead.
+// on the leader's "accumulator empty" barrier.  Measured against two 1-CTA MMAs per pair with the key tile multicast
+// to both CTAs: +0.4 % at 1088 columns, +10 % at 5120 (profiles/r01/k4_variants.md).
 // =====================================================================================
 constexpr uint32_t PEER_MASK = 0xFEFFFFFFu;        // clears the cluster-rank bit of a shared address: the even CTA
 constexpr int STAGE2_BYTES = A_BYTES + B_BYTES / 2;  // 32 KB per CTA and stage
@@ -684,30 +428,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-template <int KP, int STAGES, int CL>
-int launch_tc(kb_ctx* ctx, const CUtensorMap& tmap, const CUtensorMap& tmap_b, const TcParams& prm, int workers) {
-    using L = Smem<KP, STAGES>;
-    auto kern = k4_tc<KP, STAGES, CL>;
-    static bool attr_set[16] = {false};
-    if (!attr_set[ctx->device & 15]) {
-        KB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::TOTAL));
-        attr_set[ctx->device & 15] = true;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(workers * CL));
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = L::TOTAL;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    KB_CUDA(cudaLaunchKernelEx(&cfg, kern, tmap, tmap_b, prm));
-    ctx->launches++;
-    KB_CUDA(cudaGetLastError());
-    return KB_OK;
-}
-
 template <int KP, int STAGES, int QCAP>
 int launch_tc2(kb_ctx* ctx, const CUtensorMap& tmap, const TcParams& prm, int workers) {
     using L = Smem2<KP, STAGES, QCAP>;
@@ -732,38 +452,18 @@ int launch_tc2(kb_ctx* ctx, const CUtensorMap& tmap, const TcParams& prm, int wo
     return KB_OK;
 }
 
-// shared memory: 6 x 32 KB stages (2-CTA MMA) or 4 x 48 KB (one MMA per CTA) next to lists of up to 32 entries per
-// row; the wide lists (48, 64: n_neighbors 27..60) take the room of two stages (one for the 48 KB stages)
+// shared memory: 32 KB stages next to the lists and the insertion queues (16 entries per row = 16 KB; 12 for 16-wide
+// lists): 6 stages up to 16-wide lists, 5 for 24 / 32, 4 for 48 / 64 (n_neighbors 27..60).  Wide rows (>= 2560 columns:
+// long MMA tiles, light epilogue) with 24-wide lists trade most of the queue for the sixth stage.
 template <int KP>
-int launch_tc_kp(kb_ctx* ctx, const CUtensorMap& tmap, const CUtensorMap& tmap_b, int cl, const TcParams& prm, int workers) {
-    // 32 KB stages next to the lists and the insertion queues (16 entries per row = 16 KB; 12 for 16-wide lists):
-    // 6 stages up to 16-wide lists, 5 for 24 / 32, 4 for 48 / 64.  Wide rows (>= 2560 columns: long MMA tiles, light
-    // epilogue) with 24-wide lists trade most of the queue for the sixth stage.
+int launch_tc_kp(kb_ctx* ctx, const CUtensorMap& tmap, const TcParams& prm, int workers) {
     constexpr int ST2 = KP <= 16 ? 6 : (KP <= 32 ? 5 : 4);
     constexpr int Q2 = KP == 16 ? 12 : 16;
-    constexpr int ST1 = KP <= 32 ? 4 : 3;
-    // CTA pairs run one 2-CTA MMA (k4_tc2) unless KB_KNN_MMA2=0 asks for the two-MMA multicast kernel (experiments)
-    const char* m2 = getenv("KB_KNN_MMA2");
-    if (cl == 2 && !(m2 && atoi(m2) == 0)) {
-        if constexpr (KP == 24) { if (prm.k_blocks >= 40) return launch_tc2<24, 6, 4>(ctx, tmap, prm, workers); }
-        return launch_tc2<KP, ST2, Q2>(ctx, tmap, prm, workers);
-    }
-    if (cl == 4) return launch_tc<KP, ST1, 4>(ctx, tmap, tmap_b, prm, workers);
-    if (cl == 2) return launch_tc<KP, ST1, 2>(ctx, tmap, tmap_b, prm, workers);
-    return launch_tc<KP, ST1, 1>(ctx, tmap, tmap_b, prm, workers);
+    if constexpr (KP == 24) { if (prm.k_blocks >= 40) return launch_tc2<24, 6, 4>(ctx, tmap, prm, workers); }
+    return launch_tc2<KP, ST2, Q2>(ctx, tmap, prm, workers);
 }
 
 }  // namespace
-
-#ifdef KB_TC_STATS
-extern "C" __attribute__((visibility("default"))) int kb_debug_tc_stats(unsigned long long* out3, int reset) {
-    unsigned long long z = 0;
-    cudaMemcpyFromSymbol(&out3[0], g_tc_inserts, 8); cudaMemcpyFromSymbol(&out3[1], g_tc_cold_chunks, 8);
-    cudaMemcpyFromSymbol(&out3[2], g_tc_chunks, 8);
-    if (reset) { cudaMemcpyToSymbol(g_tc_inserts, &z, 8); cudaMemcpyToSymbol(g_tc_cold_chunks, &z, 8); cudaMemcpyToSymbol(g_tc_chunks, &z, 8); }
-    return 0;
-}
-#endif
 
 int kb_knn_tc_launch(kb_ctx* ctx, const KbKnnPlan& p, const KbTcArgs& a) {
     if (!ctx->encode_tiled) {
@@ -783,16 +483,6 @@ int kb_knn_tc_launch(kb_ctx* ctx, const KbKnnPlan& p, const KbTcArgs& a) {
                                                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                                                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS) { kb_set_error("cuTensorMapEncodeTiled failed (%d)", (int)cr); return KB_ECUDA; }
-    // key tiles arrive in parts of 128 rows (1 or 2 CTAs per cluster) or 64 rows (4 CTAs)
-    CUtensorMap tmap_b = tmap;
-    if (p.cl == 4) {
-        const cuuint32_t box_b[2] = {BK, (cuuint32_t)(BN / 4)};
-        cr = ((EncodeTiledFn)ctx->encode_tiled)(&tmap_b, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(a.d_operand),
-                                               gdim, gstride, box_b, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (cr != CUDA_SUCCESS) { kb_set_error("cuTensorMapEncodeTiled failed (%d)", (int)cr); return KB_ECUDA; }
-    }
     TcParams prm;
     prm.nk = a.nk; prm.q_row0 = a.q_row0; prm.nq = a.nq;
     prm.slots = p.slots;
@@ -804,11 +494,11 @@ int kb_knn_tc_launch(kb_ctx* ctx, const KbKnnPlan& p, const KbTcArgs& a) {
     prm.arrive = a.d_arrive; prm.epoch = a.d_epoch; prm.rows_per_src = a.rows_per_src > 0 ? a.rows_per_src : 1;
     prm.self_rank = a.self_rank;
     switch (p.kp) {
-        case 8: return launch_tc_kp<8>(ctx, tmap, tmap_b, p.cl, prm, p.workers);
-        case 16: return launch_tc_kp<16>(ctx, tmap, tmap_b, p.cl, prm, p.workers);
-        case 24: return launch_tc_kp<24>(ctx, tmap, tmap_b, p.cl, prm, p.workers);
-        case 32: return launch_tc_kp<32>(ctx, tmap, tmap_b, p.cl, prm, p.workers);
-        case 48: return launch_tc_kp<48>(ctx, tmap, tmap_b, p.cl, prm, p.workers);
-        default: return launch_tc_kp<64>(ctx, tmap, tmap_b, p.cl, prm, p.workers);
+        case 8: return launch_tc_kp<8>(ctx, tmap, prm, p.workers);
+        case 16: return launch_tc_kp<16>(ctx, tmap, prm, p.workers);
+        case 24: return launch_tc_kp<24>(ctx, tmap, prm, p.workers);
+        case 32: return launch_tc_kp<32>(ctx, tmap, prm, p.workers);
+        case 48: return launch_tc_kp<48>(ctx, tmap, prm, p.workers);
+        default: return launch_tc_kp<64>(ctx, tmap, prm, p.workers);
     }
 }

@@ -6,7 +6,7 @@
 // layout on every rank) that its peers map:
 //   * after K3 a rank pushes its shard of each gathered array into every peer's arena on a side stream (copy engines,
 //     three peers at a time), nearest-following rank first, and raises arrive[rank] = epoch there as each shard
-//     completes (KB_XCHG_SM=1 selects kx_push_sm instead: SM stores over NVLink next to the running K4 -- measured slower);
+//     completes;
 //   * K4 (kb_knn_tc.cu) starts on the local shard at once; its TMA producer polls arrive[r] before the first
 //     key tile of rank r, so the transfer overlaps the sweep tile by tile;
 //   * K5 stores its rows straight into every peer's gathered result arrays (stores over NVLink);
@@ -41,8 +41,6 @@ struct kb_xchg {
     bool attached;
     cudaStream_t extra[2];                // two more copy streams: three peer copies in flight at a time
     cudaEvent_t ev_fork, ev_join[2];
-    uint32_t* d_count;                    // per destination: CTAs of kx_push_sm that have finished its shard
-    int sm_push;                          // 1: shards are pushed by a kernel (SM stores over NVLink), 0: by the copy engines
 };
 
 namespace {
@@ -96,48 +94,6 @@ __global__ void kx_signal_arrive(const uint8_t* local, uint8_t* peer_arena, int 
     __threadfence_system();
     st_release_sys(&reinterpret_cast<KbXchgCtrl*>(peer_arena)->arrive[rank], e);
 }
-// Optional (KB_XCHG_SM=1): shards pushed by the SMs.  Every destination in turn (nearest-following rank first, the order
-// in which K4 sweeps) gets this rank's shard of every region with the WHOLE grid storing to it over NVLink; the last CTA
-// to finish a destination raises its arrival flag.  The kernel runs NEXT TO the persistent K4 CTAs (no shared memory):
-// it must never need an SM of its own.  Not the default: see kb_xchg_create.
-struct KxRegions { int n; int64_t off[4]; int64_t bytes[4]; };
-
-__global__ void __launch_bounds__(256)
-kx_push_sm(uint8_t* local, uint8_t* const* peer, int world, int rank, KxRegions rg, uint32_t* count) {
-    const KbXchgCtrl* c = reinterpret_cast<const KbXchgCtrl*>(local);
-    const uint32_t e = c->epoch;
-    const int t = threadIdx.x;
-    if (t < world && t != rank) wait_ge(&c->done[t], e - 1, 0, t);      // every peer is done with my previous shard
-    __syncthreads();
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int d = 1; d < world; ++d) {
-        const int p = (rank - d + world) % world;
-        uint8_t* dst_arena = peer[p];
-        for (int r = 0; r < rg.n; ++r) {
-            const int64_t off = rg.off[r] + (int64_t)rank * rg.bytes[r];
-            const uint4* src = reinterpret_cast<const uint4*>(local + off);
-            uint4* dst = reinterpret_cast<uint4*>(dst_arena + off);
-            const int64_t n16 = rg.bytes[r] >> 4;
-            int64_t i = (int64_t)blockIdx.x * blockDim.x + t;
-            for (; i + 3 * stride < n16; i += 4 * stride) {
-                const uint4 a = src[i], b = src[i + stride], c2 = src[i + 2 * stride], d2 = src[i + 3 * stride];
-                dst[i] = a; dst[i + stride] = b; dst[i + 2 * stride] = c2; dst[i + 3 * stride] = d2;
-            }
-            for (; i < n16; i += stride) dst[i] = src[i];
-        }
-        __threadfence_system();                               // my stores are performed at the peer before ...
-        __syncthreads();
-        if (t == 0) {
-            const uint32_t prev = atomicAdd(&count[p], 1u);   // ... this CTA is counted
-            if (prev == gridDim.x - 1) {                      // last CTA of this destination
-                count[p] = 0;                                 // (next pass; ordered by the stream)
-                __threadfence_system();
-                st_release_sys(&reinterpret_cast<KbXchgCtrl*>(dst_arena)->arrive[rank], e);
-            }
-        }
-    }
-}
-
 // my small record (rec_words u32 at rec_off + rank*rec_words*4) to every peer, then lists[rank] = epoch there
 __global__ void kx_finish(uint8_t* local, uint8_t* const* peer, int world, int rank, int64_t rec_off, int rec_words) {
     const uint32_t e = reinterpret_cast<const KbXchgCtrl*>(local)->epoch;
@@ -181,14 +137,6 @@ extern "C" int kb_xchg_create(kb_ctx* ctx, int world, int rank, int64_t bytes, k
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&x->ev_join[i], cudaEventDisableTiming);
     }
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&x->ev_fork, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&x->d_count, sizeof(uint32_t) * KB_XCHG_MAX_WORLD);
-    if (e == cudaSuccess) e = cudaMemset(x->d_count, 0, sizeof(uint32_t) * KB_XCHG_MAX_WORLD);
-    {   // KB_XCHG_SM=1: push the shards with a kernel (kx_push_sm) instead of the copy engines.  Measured on 8 x B200, 50k contigs:
-        // 0.775 ms per pass against 0.626 ms with the copy engines -- the push finishes at the same time either way (0.31-0.37 ms
-        // into the pass), but the kernel's CTAs take issue slots and L2 bandwidth from the persistent K4 CTAs they run next to.
-        const char* f = getenv("KB_XCHG_SM");
-        x->sm_push = f ? (atoi(f) != 0) : 0;
-    }
     x->peer[rank] = x->local;
     *out = x; *d_local = x->local;
     return KB_OK;
@@ -225,7 +173,6 @@ extern "C" int kb_xchg_destroy(kb_xchg* x) {
         if (p != x->rank && x->peer[p]) cudaIpcCloseMemHandle(x->peer[p]);
     for (int i = 0; i < 2; ++i) { if (x->extra[i]) cudaStreamDestroy(x->extra[i]); if (x->ev_join[i]) cudaEventDestroy(x->ev_join[i]); }
     if (x->ev_fork) cudaEventDestroy(x->ev_fork);
-    cudaFree(x->d_count);
     cudaFree(x->d_peer);
     cudaFree(x->local);
     free(x);
@@ -261,23 +208,6 @@ extern "C" int kb_xchg_begin(kb_xchg* x) {
 extern "C" int kb_xchg_push(kb_xchg* x, void* stream, int n_regions, const int64_t* region_off, const int64_t* shard_bytes) {
     KB_CHECK_ARG(x && x->attached && n_regions >= 0 && (n_regions == 0 || (region_off && shard_bytes)), "arguments");
     cudaStream_t st = (cudaStream_t)stream;
-    if (x->sm_push) {
-        KB_CHECK_ARG(n_regions <= 4, "at most 4 regions");
-        KxRegions rg; rg.n = 0;
-        for (int r = 0; r < n_regions; ++r) {
-            const int64_t off = region_off[r] + (int64_t)x->rank * shard_bytes[r];
-            KB_CHECK_ARG(off >= (int64_t)sizeof(KbXchgCtrl) && off + shard_bytes[r] <= x->bytes, "region outside the arena");
-            KB_CHECK_ARG((region_off[r] % 16) == 0 && (shard_bytes[r] % 16) == 0, "regions must be multiples of 16 bytes");
-            if (shard_bytes[r] == 0) continue;
-            rg.off[rg.n] = region_off[r]; rg.bytes[rg.n] = shard_bytes[r]; ++rg.n;
-        }
-        int ctas = 64;
-        if (const char* f = getenv("KB_XCHG_SM_CTAS")) { const int v = atoi(f); if (v >= 1 && v <= 1024) ctas = v; }
-        kx_push_sm<<<ctas, 256, 0, st>>>(x->local, x->d_peer, x->world, x->rank, rg, x->d_count);
-        x->ctx->launches++;
-        KB_CUDA(cudaGetLastError());
-        return KB_OK;
-    }
     kx_wait<<<1, KB_XCHG_MAX_WORLD, 0, st>>>(x->local, x->world, x->rank, 0);
     x->ctx->launches++;
     KB_CUDA(cudaGetLastError());

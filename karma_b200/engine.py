@@ -790,10 +790,6 @@ def profile_and_knn(engine, bases, offsets, key_len, kmer_size="5p6", n_neighbor
 # the pre-planned pass: static buffers, one enqueue, CUDA graph, peer-memory exchange
 # ---------------------------------------------------------------------------------------
 
-import os as _os
-_XCHG_DEBUG = bool(_os.environ.get("KB_XCHG_DEBUG"))
-
-
 class _KnnXchg(ctypes.Structure):
     """kb_knn_xchg of include/karma_b200.h"""
     _fields_ = [("d_arrive", c_void_p), ("d_epoch", c_void_p), ("rows_per_src", c_int64), ("n_peers", ctypes.c_int32),
@@ -1181,9 +1177,6 @@ class PassPlan:
             self.graph.replay()
         else:
             self.enqueue()
-        if _XCHG_DEBUG:
-            import sys
-            print("[karma_b200 rank %d] pass %d enqueued" % (self.rank, self._step), file=sys.stderr, flush=True)
         slot = self._step & 1
         self.h_val[slot].copy_(self.rec_all, non_blocking=True)
         self._events[slot].record(torch.cuda.current_stream(self.engine.device))

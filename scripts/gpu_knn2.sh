@@ -14,4 +14,3 @@ try:
 except Exception as e:
     print("failed", e); print(open("gpurun_out/bench.err").read()[-2500:])
 PY
-timeout 300 python scripts/exp_k4.py 5p6 2 1,2,4,8 2>&1 | grep "K4 "

@@ -113,27 +113,22 @@ def test_header_is_plain_c_and_a_c_host_links(lib, tmp_path):
         assert run.returncode != 0 and "no CPU fallback" in run.stderr, run.stdout + run.stderr
 
 
-def test_knn_plan_workspace_bounds(lib, monkeypatch):
+def test_knn_plan_workspace_bounds(lib):
     """kb_knn_workspace_bytes (host only) over the shapes of BASELINE.json and the shard shapes of 2-8 GPUs:
-    the plan never asks for more candidate slots than K5 can merge (512 per row), for every cluster variant."""
+    the plan never asks for more candidate slots than K5 can merge (512 per row)."""
     from karma_b200 import _lib
     shapes = [(1000, 1000, 0), (50000, 50000, 0), (6250, 50000, 18750), (62500, 500000, 62500), (125000, 1000000, 0),
               (250000, 2000000, 1750000), (130, 130, 0), (513, 513, 0)]
-    for cluster in (None, "1", "2", "4"):
-        if cluster is None:
-            monkeypatch.delenv("KB_KNN_CLUSTER", raising=False)
-        else:
-            monkeypatch.setenv("KB_KNN_CLUSTER", cluster)
-        for nq, nk, q0 in shapes:
-            for dp in (1088, 5120):
-                for k in (2, 10, 15, 24, 40, 60):
-                    kp = 8 if k <= 2 else 16 if k <= 10 else 24 if k <= 18 else 32 if k <= 26 else 48 if k <= 42 else 64
-                    for impl in (_lib.KB_KNN_SIMT, _lib.KB_KNN_TC):
-                        b = lib.kb_knn_workspace_bytes(None, nq, nk, q0, dp, k, impl, 0)
-                        lo = nq * kp * 8 + nq * 4 + nq * 4                       # one list of candidates + row bounds + uncertified rows
-                        hi = nq * 512 * 8 + nq * 8 + 8 * 256                     # at most 512 candidates per row
-                        assert lo <= b <= hi, (cluster, nq, nk, k, impl, b, lo, hi)
-                        assert lib.kb_knn_workspace_bytes(None, nq, nk, q0, dp, k, impl, 7) > b    # flagged rows add the fp64 side lists
+    for nq, nk, q0 in shapes:
+        for dp in (1088, 5120):
+            for k in (2, 10, 15, 24, 40, 60):
+                kp = 8 if k <= 2 else 16 if k <= 10 else 24 if k <= 18 else 32 if k <= 26 else 48 if k <= 42 else 64
+                for impl in (_lib.KB_KNN_SIMT, _lib.KB_KNN_TC):
+                    b = lib.kb_knn_workspace_bytes(None, nq, nk, q0, dp, k, impl, 0)
+                    lo = nq * kp * 8 + nq * 4 + nq * 4                       # one list of candidates + row bounds + uncertified rows
+                    hi = nq * 512 * 8 + nq * 8 + 8 * 256                     # at most 512 candidates per row
+                    assert lo <= b <= hi, (nq, nk, k, impl, b, lo, hi)
+                    assert lib.kb_knn_workspace_bytes(None, nq, nk, q0, dp, k, impl, 7) > b    # flagged rows add the fp64 side lists
 
 
 def _plan(lib, nq, nk, q0, dp, k, sm=148):
@@ -144,8 +139,7 @@ def _plan(lib, nq, nk, q0, dp, k, sm=148):
     pieces = np.zeros((info["pieces"], 8), dtype=np.int32)
     start = np.zeros(info["workers"] + 1, dtype=np.int32)
     m_blocks = -(-nq // 128)
-    cl = 2 if m_blocks >= 2 else 1
-    groups = -(-m_blocks // cl)
+    groups = -(-m_blocks // 2)                                            # CTA pairs, also for a lone query block
     slots = np.zeros(groups, dtype=np.int32)
     vp = ctypes.c_void_p
     assert lib.kb_knn_plan_table(sm, 2, nq, nk, q0, dp, k, pieces.ctypes.data_as(vp), start.ctypes.data_as(vp),
@@ -159,7 +153,7 @@ def _plan(lib, nq, nk, q0, dp, k, sm=148):
                                            (257, 700, 300, 1088, 5), (1, 600, 599, 64, 1)])
 def test_knn_piece_table_covers_every_tile_once(lib, nq, nk, q0, dp, k):
     """The host-built schedule of the tensor kernel (kb_knn.cuh: KbPiece): every (query group, key tile) pair is
-    visited exactly once, every piece has a candidate slot of its own, and the busiest cluster carries at most
+    visited exactly once, every piece has a candidate slot of its own, and the busiest CTA pair carries at most
     a few tile visits more than the mean (SURVEY 8e: small shards must keep all 74 CTA pairs busy)."""
     import numpy as np
     info, pieces, start, slots, groups = _plan(lib, nq, nk, q0, dp, k)

@@ -89,15 +89,17 @@ def test_tensor_core_gram_is_exact(engine):
 
 
 def test_query_shard_equals_full(engine):
-    """Multi-GPU layout on one GPU: a query-row shard against all keys gives the same rows."""
+    """Multi-GPU layout on one GPU: a query-row shard against all keys gives the same rows, also for a lone
+    query block (at most 128 rows: a CTA pair whose second CTA has no live rows), the last one ending at the last key."""
     asm = synth.s1_families(1000, seed=31)
     mode = mode_of("5p6")
     d_bases, d_offsets, d_len = engine.upload(asm.bases, asm.offsets, asm.key_len)
     counts, _, _ = engine.count(d_bases, d_offsets, asm.n, mode)
     _, operand, rowmeta = engine.normalise(counts, 1088, d_len, want_profile=False)
     full_i, full_d, _ = engine.knn(operand, rowmeta, 5, impl=_lib.KB_KNN_TC)
-    part_i, part_d, _ = engine.knn(operand, rowmeta, 5, q_row0=250, nq=333, impl=_lib.KB_KNN_TC)
-    assert torch.equal(full_i[250:583], part_i) and torch.equal(full_d[250:583], part_d)
+    for q0, nq in ((250, 333), (250, 100), (0, 1), (872, 128)):
+        part_i, part_d, _ = engine.knn(operand, rowmeta, 5, q_row0=q0, nq=nq, impl=_lib.KB_KNN_TC)
+        assert torch.equal(full_i[q0:q0 + nq], part_i) and torch.equal(full_d[q0:q0 + nq], part_d), (q0, nq)
 
 
 def test_full_size_knn_properties_50k(engine):
