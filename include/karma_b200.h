@@ -416,15 +416,43 @@ KB_API int kb_umap_layout(kb_ctx* ctx, int64_t n, int64_t nnz, const int64_t* d_
                    int32_t dim, int32_t n_epochs, double a, double b, double gamma, double initial_alpha,
                    double negative_sample_rate, uint64_t seed, float* d_embedding, int64_t* d_samples, int64_t* nnz_kept);
 
+/* ---- K9: HDBSCAN's mutual-reachability MST (device) and its clusters (host) ----
+ * Replaces hdbscan.HDBSCAN(min_cluster_size=m).fit(embedding) of hdbscan 0.8.22 (kmer.py:296-301), metric euclidean,
+ * alpha 1, eom selection; the reference of record is scikit-learn 1.9.0's port of its tree code (rules frozen in
+ * oracle/hdbscan_oracle.py).  d(i, j) = RN(sqrt(sum_c (x_ic - x_jc)^2)) in fp64 from the float32 coordinates, in
+ * coordinate order, no FMA; core_i = the core_k-th smallest of {d(i, j) : all j}, d(i, i) = 0 and duplicates counted
+ * (hdbscan's min_samples = m is core_k = m + 1); w(i, j) = max(core_i, core_j, d(i, j)).  Edges are totally ordered
+ * by (w, min(i, j), max(i, j)), so the MST is unique: it is the exact MST (hdbscan 0.8.22 defaults to an approximate
+ * one), whatever the execution order.
+ * kb_hdbscan_mst (device pointers; Boruvka over the implicit complete graph, one host read per round):
+ *  d_x       float[n*dim]   the points, row-major, finite (KB_EINVAL otherwise); n >= 2
+ *  dim       1..64, core_k 1..min(n, 128) (KB_EINVAL below 1 or above n, KB_EUNSUPPORTED above 64 / 128)
+ *  d_core    double[n]      out: core distances
+ *  d_edges   int32[(n-1)*2] out: the MST's edges, each (min, max), sorted by (w, min, max)
+ *  d_weights double[n-1]    out: their weights
+ * Synchronises once per round; the sorted edges are enqueued on the context stream when it returns.
+ * kb_hdbscan_labels (host pointers, no GPU): scikit-learn's make_single_linkage, _condense_tree, _compute_stability,
+ * _get_clusters (eom, allow_single_cluster), _do_labelling and get_probabilities over such a sorted spanning tree,
+ * with their fp64 operation order.  KB_EINVAL for an index outside [0, n), an edge not (min, max), edges out of
+ * (w, min, max) order, a negative or non-finite weight, a cycle, or min_cluster_size < 2.
+ *  labels int32[n] (-1 = noise; clusters numbered in the order of their condensed-tree ids), probabilities double[n],
+ *  n_clusters out.  It also returns KB_EINVAL, with a message naming an internal inconsistency, if its own tree walk
+ *  contradicts itself; a valid tree never does. */
+KB_API int kb_hdbscan_mst(kb_ctx* ctx, int64_t n, int32_t dim, const float* d_x, int32_t core_k,
+                   double* d_core, int32_t* d_edges /* [n-1][2], (min,max) */, double* d_weights /* [n-1] */);
+KB_API int kb_hdbscan_labels(int64_t n, const int32_t* edges, const double* weights, int32_t min_cluster_size,
+                   int32_t allow_single_cluster, int32_t* labels, double* probabilities, int64_t* n_clusters);
+
 /* Per-stage device times.  With timing enabled every launch of a stage is bracketed
  * by a CUDA-event pair on the context stream (a ring of 128 pairs per stage).
  * kb_stage_ms synchronises, returns the mean duration (ms) and the number of launches
  * recorded since the last read, and resets the stage.
  *  which: 0 count, 1 count-long, 2 compact, 3 normalise, 4 knn-gemm, 5 rerank, 6 exact side path,
- *         7 read-graph build, 8 group-pair connection weights */
+ *         7 read-graph build, 8 group-pair connection weights, 9 K9 core distances, 10 K9 Boruvka rounds (one launch
+ *         recorded per round), 11 K9 edge sort */
 KB_API int kb_enable_timing(kb_ctx* ctx, int on);
 KB_API int kb_stage_ms(kb_ctx* ctx, int which, float* mean_ms, int* n_launches);
-/* Number of kernels this library launched since the context was created. */
+/* Number of kernels this library launched since the context was created (a CUB device-wide call counts as one). */
 KB_API int64_t kb_launch_count(kb_ctx* ctx);
 
 #ifdef __cplusplus

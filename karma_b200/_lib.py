@@ -17,7 +17,8 @@ KB_KNN_AUTO, KB_KNN_SIMT, KB_KNN_TC = 0, 1, 2
 KB_EINVAL, KB_ENOGPU, KB_EUNSUPPORTED = -1, -3, -4
 KB_COUNT_NO_COLUMNS = 0x100
 
-STAGES = {"count": 0, "count_long": 1, "compact": 2, "normalise": 3, "knn_gemm": 4, "rerank": 5, "knn_exact": 6, "readgraph": 7, "links": 8}
+STAGES = {"count": 0, "count_long": 1, "compact": 2, "normalise": 3, "knn_gemm": 4, "rerank": 5, "knn_exact": 6, "readgraph": 7, "links": 8,
+          "hdbscan_core": 9, "hdbscan_mst": 10, "hdbscan_sort": 11}
 
 
 def KB_MODE_K(k):
@@ -81,6 +82,8 @@ SIGNATURES = {
     "kb_fuzzy_graph_fetch": (c_int, [_P, _P, _P, _P]),
     "kb_umap_layout": (c_int, [_P, c_int64, c_int64, _P, _P, _P, c_int32, c_int32, c_double, c_double, c_double, c_double, c_double,
                                c_uint64, _P, _P, POINTER(c_int64)]),
+    "kb_hdbscan_mst": (c_int, [_P, c_int64, c_int32, _P, c_int32, _P, _P, _P]),
+    "kb_hdbscan_labels": (c_int, [c_int64, _P, _P, c_int32, c_int32, _P, _P, POINTER(c_int64)]),
     "kb_enable_timing": (c_int, [_P, c_int]),
     "kb_stage_ms": (c_int, [_P, c_int, POINTER(c_float), POINTER(c_int)]),
     "kb_launch_count": (c_int64, [_P]),

@@ -35,7 +35,7 @@ int kb_mode_describe(int mode, KbMode* m) {
     return KB_OK;
 }
 
-extern "C" int kb_version(void) { return 102; }
+extern "C" int kb_version(void) { return 103; }
 extern "C" const char* kb_last_error(void) { return g_err; }
 
 extern "C" int kb_mode_columns(int mode) {

@@ -8,7 +8,7 @@
 #include <nvtx3/nvToolsExt.h>          // header-only (NVTX v3): ranges are no-ops unless a profiler is attached
 #include "../../include/karma_b200.h"
 
-#define KB_N_TIMERS 9
+#define KB_N_TIMERS 12
 #define KB_EV_RING 128
 
 struct kb_ctx {
@@ -63,7 +63,8 @@ int kb_cuda_fail(cudaError_t e, const char* what);
 // with timing enabled, a CUDA-event pair on the launching stream.
 static const char* const kb_stage_names[KB_N_TIMERS] = {
     "kb:K1 count", "kb:K1 count (split contigs)", "kb:K2 compact", "kb:K3 normalise", "kb:K4 distance GEMM + top-k",
-    "kb:K5 merge + exact rerank", "kb:K4x/K6 exact distances", "kb:read graph", "kb:group links"};
+    "kb:K5 merge + exact rerank", "kb:K4x/K6 exact distances", "kb:read graph", "kb:group links",
+    "kb:K9 core distances", "kb:K9 Boruvka round", "kb:K9 edge sort"};
 struct KbTimer {
     kb_ctx* c; int which; int slot;
     KbTimer(kb_ctx* ctx, int w) : c(ctx), which(w), slot(0) {
