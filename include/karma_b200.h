@@ -443,13 +443,57 @@ KB_API int kb_hdbscan_mst(kb_ctx* ctx, int64_t n, int32_t dim, const float* d_x,
 KB_API int kb_hdbscan_labels(int64_t n, const int32_t* edges, const double* weights, int32_t min_cluster_size,
                    int32_t allow_single_cluster, int32_t* labels, double* probabilities, int64_t* n_clusters);
 
+/* ---- K10: UMAP's spectral initialisation over the pruned fuzzy graph (the stage between K7 and K8) ----
+ * Replaces umap.spectral.spectral_layout of umap-learn 0.3.9 (init="spectral"), disconnected graphs included (rules
+ * frozen in oracle/umap_spectral_oracle.py).  The graph (as for kb_umap_layout: indptr from 0 to nnz, indices in
+ * [0, n), data finite and > 0, else KB_EINVAL; symmetric, as K7 builds it) is pruned with K8's rule, w >= max / n_epochs
+ * (n_epochs 0: no pruning, for a graph pruned already).  Its weakly connected components are labelled in the order of
+ * their smallest vertex (scipy's connected_components).
+ *  - A connected graph, and every component of at least 2 * dim vertices of a disconnected one, is solved: the unit
+ *    eigenvectors of the dim smallest non-trivial eigenvalues of L = I - D^-1/2 W D^-1/2, each with its largest-|.|
+ *    entry positive.  fp64 Lanczos with full reorthogonalisation and thick restart on D^-1/2 W D^-1/2, the trivial
+ *    vector D^1/2 1 deflated; every returned Ritz pair has a residual estimate ||M v - theta v|| <= 1e-9.  A solve that
+ *    needs more than 500 restarts leaves its component not converged (status 2: umap's ARPACK fallback, a draw); a
+ *    repeated wanted eigenvalue (a uniform ring, a clique) is found only through rounding and may end so.
+ *  - Components of fewer than 2 * dim vertices take uniform draws (status 0).
+ *  - Meta points (n_comp > 1): with n_comp > 2 * dim, scikit-learn 1.9.0's spectral embedding of the components'
+ *    float32 centroids (numpy's float32 mean, bit for bit) under exp(-d^2), over its global max; this needs the data
+ *    (KB_EINVAL without), refuses more than 65536 components (KB_EUNSUPPORTED: n_comp^2 fp64 of dense affinity), and
+ *    an affinity that underflows to 0 (KB_EUNSUPPORTED); a meta solve that does not converge is KB_EINVAL.  With
+ *    2 <= n_comp <= 2 * dim, the rows of [eye(k), 0; -eye(k), 0], k = ceil(n_comp / 2).
+ *  - range[c] = half the smallest positive euclidean distance from meta point c to the others, fp64 in coordinate
+ *    order without FMA (umap takes it from a dot-product expansion; DESIGN §3 K10); 10 for a connected graph.
+ * The same inputs give the same bits: fixed-order reductions, integer atomics only.
+ * kb_spectral_build (device pointers; synchronises; keeps the result in the context until the next build):
+ *  dim      1..64 (KB_EUNSUPPORTED above); a connected graph needs n > dim + 1 (KB_EINVAL)
+ *  d_x      nullable: the data, row-major n x x_cols, x_dtype 1 float32 or 2 float64 (every value is cast to
+ *           float32 first, as umap's check_array does; not finite -> KB_EINVAL); x_dtype 0: none
+ *  n_comp   out: the number of components
+ * kb_spectral_fetch (any pointer may be NULL): h_size int32[n_comp], h_status int32[n_comp] (0 draw, 1 solved,
+ *  2 not converged), h_range double[n_comp], h_stats int64[6] (Lanczos steps and restarts over the components, the
+ *  meta solve's steps and restarts, component rounds, 0); device copies enqueued on the context stream: d_labels
+ *  int32[n], d_meta double[n_comp*dim] (n_comp > 1), d_vectors double[n*dim] (row i: vertex i's entries of its
+ *  component's vectors; zero where not solved), d_centroids double[n_comp*x_cols] (n_comp > 2 * dim).
+ * kb_spectral_assemble: the float32 [n, dim] layout spectral_layout returns, with umap's arithmetic: solved,
+ *  fp32(v * (range / max|v|) + meta) (fp32(v) when connected); otherwise fp32((-range + 2 range u) + meta) (no meta
+ *  when connected), u = d_u[i*dim + d], the uniform [0, 1) draws of random_state.uniform for vertex i's component,
+ *  row i = vertex i (d_u may be NULL when every component is solved).  Enqueued on the context stream. */
+KB_API int kb_spectral_build(kb_ctx* ctx, int64_t n, int64_t nnz, const int64_t* d_indptr, const int32_t* d_indices,
+                   const double* d_data, int32_t n_epochs, int32_t dim, const void* d_x, int32_t x_dtype, int64_t x_cols,
+                   int64_t* n_comp);
+KB_API int kb_spectral_fetch(kb_ctx* ctx, int32_t* h_size, int32_t* h_status, double* h_range, int64_t* h_stats,
+                   int32_t* d_labels, double* d_meta, double* d_vectors, double* d_centroids);
+KB_API int kb_spectral_assemble(kb_ctx* ctx, const double* d_u, float* d_out);
+
 /* Per-stage device times.  With timing enabled every launch of a stage is bracketed
  * by a CUDA-event pair on the context stream (a ring of 128 pairs per stage).
  * kb_stage_ms synchronises, returns the mean duration (ms) and the number of launches
  * recorded since the last read, and resets the stage.
  *  which: 0 count, 1 count-long, 2 compact, 3 normalise, 4 knn-gemm, 5 rerank, 6 exact side path,
  *         7 read-graph build, 8 group-pair connection weights, 9 K9 core distances, 10 K9 Boruvka rounds (one launch
- *         recorded per round), 11 K9 edge sort */
+ *         recorded per round), 11 K9 edge sort, 12 K10 components (validation, pruning, component rounds, labels and
+ *         the permuted CSR), 13 K10 eigensolve (every component solve, host Ritz steps included), 14 K10 meta-embedding
+ *         (centroids, affinity, the meta solve, data ranges) */
 KB_API int kb_enable_timing(kb_ctx* ctx, int on);
 KB_API int kb_stage_ms(kb_ctx* ctx, int which, float* mean_ms, int* n_launches);
 /* Number of kernels this library launched since the context was created (a CUB device-wide call counts as one). */

@@ -35,7 +35,7 @@ int kb_mode_describe(int mode, KbMode* m) {
     return KB_OK;
 }
 
-extern "C" int kb_version(void) { return 103; }
+extern "C" int kb_version(void) { return 104; }
 extern "C" const char* kb_last_error(void) { return g_err; }
 
 extern "C" int kb_mode_columns(int mode) {
@@ -90,6 +90,7 @@ extern "C" int kb_destroy(kb_ctx* c) {
     kb_links_free(c);
     kb_fuzzy_free(c);
     kb_knn_cache_free(c);
+    kb_spectral_free(c);
     if (c->pool) { cudaDeviceSynchronize(); cudaMemPoolDestroy(c->pool); }
     free(c);
     return KB_OK;

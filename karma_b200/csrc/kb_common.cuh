@@ -8,7 +8,7 @@
 #include <nvtx3/nvToolsExt.h>          // header-only (NVTX v3): ranges are no-ops unless a profiler is attached
 #include "../../include/karma_b200.h"
 
-#define KB_N_TIMERS 12
+#define KB_N_TIMERS 15
 #define KB_EV_RING 128
 
 struct kb_ctx {
@@ -43,6 +43,8 @@ struct kb_ctx {
     void* encode_tiled;
     // kNN plans and uploaded piece tables (kb_knn.cu)
     void* knn_cache;
+    // the spectral initialisation of the last kb_spectral_build (kb_spectral.cu, owned)
+    void* spectral;
 };
 
 void kb_set_error(const char* fmt, ...);
@@ -64,7 +66,8 @@ int kb_cuda_fail(cudaError_t e, const char* what);
 static const char* const kb_stage_names[KB_N_TIMERS] = {
     "kb:K1 count", "kb:K1 count (split contigs)", "kb:K2 compact", "kb:K3 normalise", "kb:K4 distance GEMM + top-k",
     "kb:K5 merge + exact rerank", "kb:K4x/K6 exact distances", "kb:read graph", "kb:group links",
-    "kb:K9 core distances", "kb:K9 Boruvka round", "kb:K9 edge sort"};
+    "kb:K9 core distances", "kb:K9 Boruvka round", "kb:K9 edge sort", "kb:K10 components", "kb:K10 eigensolve",
+    "kb:K10 meta-embedding"};
 struct KbTimer {
     kb_ctx* c; int which; int slot;
     KbTimer(kb_ctx* ctx, int w) : c(ctx), which(w), slot(0) {
@@ -97,6 +100,7 @@ int kb_launch_count_kernels(kb_ctx* ctx, const KbMode& m, const uint8_t* d_bases
 void kb_links_free(kb_ctx* c);
 void kb_fuzzy_free(kb_ctx* c);
 void kb_knn_cache_free(kb_ctx* c);
+void kb_spectral_free(kb_ctx* c);
 // host-side file input shared by the FASTA and eq_classes parsers (kb_fasta.cu)
 int64_t kb_host_threads();
 int kb_host_read_file(const char* path, uint8_t** img, int64_t* size);
@@ -114,3 +118,82 @@ struct PoolBuf {
 };
 
 static inline int64_t kb_round_up(int64_t x, int64_t m) { return (x + m - 1) / m * m; }
+
+// ---- a fuzzy graph's CSR rows, checked as K8 and K10 check them ----
+constexpr unsigned KB_CSR_BAD_INDPTR = 1u, KB_CSR_BAD_INDEX = 2u, KB_CSR_BAD_DATA = 4u;
+
+__device__ __forceinline__ bool kb_csr_row(const int64_t* __restrict__ indptr, int64_t r, int64_t nnz, int64_t* lo, int64_t* hi) {
+    *lo = indptr[r];
+    *hi = indptr[r + 1];
+    return *lo >= 0 && *lo <= *hi && *hi <= nnz;
+}
+
+__device__ __forceinline__ bool kb_weight_ok(double w) { return w > 0.0 && w <= 1.7976931348623157e308; }
+
+// thread per row: indptr monotone from 0 to nnz, indices in [0, n), data finite and > 0 (KB_CSR_BAD_* into *flags); the
+// largest weight into *wmax_bits (atomicMax on the bits of a positive double, order-free).  No read beyond nnz entries.
+static __global__ void kb_csr_check(const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                                    const double* __restrict__ data, int64_t n, int64_t nnz,
+                                    unsigned long long* __restrict__ flags, unsigned long long* __restrict__ wmax_bits) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n) return;
+    unsigned f = 0;
+    if (r == 0 && (indptr[0] != 0 || indptr[n] != nnz)) f |= KB_CSR_BAD_INDPTR;
+    int64_t lo, hi;
+    double mx = 0.0;
+    if (!kb_csr_row(indptr, r, nnz, &lo, &hi)) {
+        f |= KB_CSR_BAD_INDPTR;
+    } else {
+        for (int64_t e = lo; e < hi; ++e) {
+            const int32_t c = indices[e];
+            if (c < 0 || (int64_t)c >= n) f |= KB_CSR_BAD_INDEX;
+            const double w = data[e];
+            if (!kb_weight_ok(w)) f |= KB_CSR_BAD_DATA;
+            else if (w > mx) mx = w;
+        }
+    }
+    if (f) atomicOr(flags, (unsigned long long)f);
+    if (mx > 0.0) atomicMax(wmax_bits, (unsigned long long)__double_as_longlong(mx));
+}
+
+// ---- hooking union-find over components (K9's Boruvka rounds, K10's connected components) ----
+// comp[i] is i's component, named by its root vertex (comp[c] == c); comp_key[c] is the edge (min << 32 | max) along which
+// component c hooks, ~0 for none.  With every component hooking along its minimum edge under one strict total order, the
+// successor graph is a forest whose only cycles are pairs that chose the same edge.
+__device__ __forceinline__ unsigned long long hd_key(int64_t a, int64_t b) {
+    return a < b ? ((unsigned long long)a << 32) | (unsigned long long)b : ((unsigned long long)b << 32) | (unsigned long long)a;
+}
+
+// each component's successor: the component at the other end of its edge (itself when it has none)
+static __global__ void hd_hook(const int32_t* __restrict__ comp, const unsigned long long* __restrict__ comp_key,
+                               int32_t* __restrict__ succ, int64_t n) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n || comp[c] != c) return;
+    const unsigned long long key = comp_key[c];
+    if (key == ~0ull) { succ[c] = (int32_t)c; return; }
+    const int32_t ca = comp[key >> 32], cb = comp[key & 0xffffffffull];
+    succ[c] = ca == c ? cb : ca;
+}
+
+// one pointer-jumping step over the components' parents; every value written is an ancestor, so concurrent reads are safe
+static __global__ void hd_jump(const int32_t* __restrict__ comp, int32_t* par, int64_t n) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n || comp[c] != c) return;
+    par[c] = par[par[c]];
+}
+
+// comp[i] <- its root; *n_comp counts the roots
+static __global__ void hd_relabel(int32_t* __restrict__ comp, const int32_t* __restrict__ par, int64_t n,
+                                  unsigned long long* __restrict__ n_comp) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int32_t c = comp[i];
+    const int32_t r = par[c];
+    comp[i] = r;
+    if (c == i && r == i) atomicAdd(n_comp, 1ull);
+}
+
+static __global__ void hd_iota(int32_t* __restrict__ comp, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) comp[i] = (int32_t)i;
+}

@@ -22,7 +22,7 @@
 //              RN(sqrt(d^2)) >= best): both skips provably leave the fp64 w of every kept candidate unchanged.
 //              atomicMin of the weight bits per component (non-negative doubles order like their bits)
 //   hd_comp_key  rows whose weight is their component's minimum: atomicMin of the key (min << 32 | max)
-//   hd_hook    each component's successor: the component at the other end of its minimum edge
+//   hd_hook    (kb_common.cuh) each component's successor: the component at the other end of its minimum edge
 //   hd_link    the only cycles are pairs choosing the same edge: the smaller id becomes a root, the other appends it
 //   hd_jump    pointer jumping to the roots, hd_relabel: comp[i] <- root, count the components
 //   edge sort  two stable CUB radix sorts: by (min << 32 | max), then by the weight bits -> (w, min, max)
@@ -158,25 +158,12 @@ __global__ void __launch_bounds__(HD_THREADS) hd_round(const float* __restrict__
     atomicMin(&comp_w[mi], (unsigned long long)__double_as_longlong(bw));
 }
 
-__device__ __forceinline__ unsigned long long hd_key(int64_t a, int64_t b) {
-    return a < b ? ((unsigned long long)a << 32) | (unsigned long long)b : ((unsigned long long)b << 32) | (unsigned long long)a;
-}
-
 __global__ void hd_comp_key(const double* __restrict__ row_w, const int32_t* __restrict__ row_j, const int32_t* __restrict__ comp,
                             const unsigned long long* __restrict__ comp_w, unsigned long long* __restrict__ comp_key, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int32_t c = comp[i];
     if ((unsigned long long)__double_as_longlong(row_w[i]) == comp_w[c]) atomicMin(&comp_key[c], hd_key(i, row_j[i]));
-}
-
-__global__ void hd_hook(const int32_t* __restrict__ comp, const unsigned long long* __restrict__ comp_key,
-                        int32_t* __restrict__ succ, int64_t n) {
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= n || comp[c] != c) return;
-    const unsigned long long key = comp_key[c];
-    const int32_t ca = comp[key >> 32], cb = comp[key & 0xffffffffull];
-    succ[c] = ca == c ? cb : ca;
 }
 
 __global__ void hd_link(const int32_t* __restrict__ comp, const int32_t* __restrict__ succ, int32_t* __restrict__ par,
@@ -196,22 +183,6 @@ __global__ void hd_link(const int32_t* __restrict__ comp, const int32_t* __restr
     edge_w[pos] = comp_w[c];
 }
 
-// one pointer-jumping step over the components' parents; every value written is an ancestor, so concurrent reads are safe
-__global__ void hd_jump(const int32_t* __restrict__ comp, int32_t* par, int64_t n) {
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= n || comp[c] != c) return;
-    par[c] = par[par[c]];
-}
-
-__global__ void hd_relabel(int32_t* __restrict__ comp, const int32_t* __restrict__ par, int64_t n, HdStatus* __restrict__ st) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const int32_t c = comp[i];
-    const int32_t r = par[c];
-    comp[i] = r;
-    if (c == i && r == i) atomicAdd(&st->n_comp, 1ull);
-}
-
 __global__ void hd_unpack(const unsigned long long* __restrict__ key, const unsigned long long* __restrict__ wbits, int64_t m,
                           int32_t* __restrict__ edges, double* __restrict__ weights) {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -219,11 +190,6 @@ __global__ void hd_unpack(const unsigned long long* __restrict__ key, const unsi
     edges[2 * e] = (int32_t)(key[e] >> 32);
     edges[2 * e + 1] = (int32_t)(key[e] & 0xffffffffull);
     weights[e] = __longlong_as_double((long long)wbits[e]);
-}
-
-__global__ void hd_iota(int32_t* __restrict__ comp, int64_t n) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) comp[i] = (int32_t)i;
 }
 
 template <int DMAX>
@@ -304,7 +270,7 @@ extern "C" int kb_hdbscan_mst(kb_ctx* ctx, int64_t n, int32_t dim, const float* 
                                                  comp_w.as<unsigned long long>(), comp_key.as<unsigned long long>(),
                                                  ek.as<unsigned long long>(), ew.as<unsigned long long>(), n, d_st);
             for (int s = 0; s < jumps; ++s) hd_jump<<<flat_blocks, 256, 0, st>>>(comp.as<int32_t>(), par.as<int32_t>(), n);
-            hd_relabel<<<flat_blocks, 256, 0, st>>>(comp.as<int32_t>(), par.as<int32_t>(), n, d_st);
+            hd_relabel<<<flat_blocks, 256, 0, st>>>(comp.as<int32_t>(), par.as<int32_t>(), n, &d_st->n_comp);
             ctx->launches += 5 + jumps;
         }
         KB_CUDA(cudaGetLastError());

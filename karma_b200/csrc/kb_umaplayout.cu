@@ -15,7 +15,7 @@
 //     on the order the atomics land in; then Y <- fp32(fp64(Y) + acc * 2^-32) and acc <- 0.
 // GPU formulation:
 //   0. before the one host synchronisation (thread per row; no read beyond the caller's nnz entries):
-//      ul_rows_check  indptr monotone from 0 to nnz, indices in [0, N), data finite and > 0, row max -> fp64 max (atomicMax
+//      kb_csr_check   indptr monotone from 0 to nnz, indices in [0, N), data finite and > 0, row max -> fp64 max (atomicMax
 //                     on the bits of a positive double, order-free);  ul_check_init: init finite
 //      ul_rows_keep   kept edges per row (w >= max / n_epochs, umap's pruning), total degree of every vertex
 //      ul_max_degree  the largest total degree, for the fixed-point range check
@@ -31,7 +31,7 @@ namespace {
 
 constexpr int UL_THREADS = 128;
 constexpr int UL_CHUNK = 16;
-constexpr unsigned UL_BAD_INDPTR = 1u, UL_BAD_INDEX = 2u, UL_BAD_DATA = 4u, UL_BAD_INIT = 8u;
+constexpr unsigned UL_BAD_INIT = 8u;     // above kb_csr_check's KB_CSR_BAD_* bits
 
 struct UlStatus {                 // device word block read back by the one host synchronisation
     unsigned long long flags;
@@ -52,38 +52,6 @@ __host__ __device__ __forceinline__ uint64_t ul_mix64(uint64_t z) {
     z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
     z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
     return z ^ (z >> 31);
-}
-
-__device__ __forceinline__ bool ul_row(const int64_t* __restrict__ indptr, int64_t r, int64_t nnz, int64_t* lo, int64_t* hi) {
-    *lo = indptr[r];
-    *hi = indptr[r + 1];
-    return *lo >= 0 && *lo <= *hi && *hi <= nnz;
-}
-
-__device__ __forceinline__ bool ul_weight_ok(double w) { return w > 0.0 && w <= 1.7976931348623157e308; }
-
-__global__ void __launch_bounds__(UL_THREADS) ul_rows_check(const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
-                                                            const double* __restrict__ data, int64_t n, int64_t nnz,
-                                                            UlStatus* __restrict__ st) {
-    const int64_t r = (int64_t)blockIdx.x * UL_THREADS + threadIdx.x;
-    if (r >= n) return;
-    unsigned f = 0;
-    if (r == 0 && (indptr[0] != 0 || indptr[n] != nnz)) f |= UL_BAD_INDPTR;
-    int64_t lo, hi;
-    double mx = 0.0;
-    if (!ul_row(indptr, r, nnz, &lo, &hi)) {
-        f |= UL_BAD_INDPTR;
-    } else {
-        for (int64_t e = lo; e < hi; ++e) {
-            const int32_t c = indices[e];
-            if (c < 0 || (int64_t)c >= n) f |= UL_BAD_INDEX;
-            const double w = data[e];
-            if (!ul_weight_ok(w)) f |= UL_BAD_DATA;
-            else if (w > mx) mx = w;
-        }
-    }
-    if (f) atomicOr(&st->flags, (unsigned long long)f);
-    if (mx > 0.0) atomicMax(&st->wmax_bits, (unsigned long long)__double_as_longlong(mx));
 }
 
 __global__ void ul_check_init(const float* __restrict__ y, int64_t total, UlStatus* __restrict__ st) {
@@ -107,11 +75,11 @@ __global__ void __launch_bounds__(UL_THREADS) ul_rows_keep(const int64_t* __rest
     if (r < n) {
         const double thr = ul_threshold(st, n_epochs);
         int64_t lo, hi;
-        if (ul_row(indptr, r, nnz, &lo, &hi)) {
+        if (kb_csr_row(indptr, r, nnz, &lo, &hi)) {
             for (int64_t e = lo; e < hi; ++e) {
                 const int32_t c = indices[e];
                 const double w = data[e];
-                if (c < 0 || (int64_t)c >= n || !ul_weight_ok(w) || w < thr) continue;
+                if (c < 0 || (int64_t)c >= n || !kb_weight_ok(w) || w < thr) continue;
                 ++kept;
                 atomicAdd(&degree[c], 1);
             }
@@ -312,7 +280,7 @@ extern "C" int kb_umap_layout(kb_ctx* ctx, int64_t n, int64_t nnz, const int64_t
     const unsigned row_blocks = (unsigned)((n + UL_THREADS - 1) / UL_THREADS);
     const int64_t total = n * dim;
     const unsigned flat_blocks = (unsigned)std::min<int64_t>((total + 255) / 256, (int64_t)ctx->sm_count * 16);
-    ul_rows_check<<<row_blocks, UL_THREADS, 0, st>>>(d_indptr, d_indices, d_data, n, nnz, d_st);
+    kb_csr_check<<<row_blocks, UL_THREADS, 0, st>>>(d_indptr, d_indices, d_data, n, nnz, &d_st->flags, &d_st->wmax_bits);
     ul_check_init<<<flat_blocks, 256, 0, st>>>(d_embedding, total, d_st);
     ul_rows_keep<<<row_blocks, UL_THREADS, 0, st>>>(d_indptr, d_indices, d_data, n, nnz, n_epochs, d_st, row_kept.as<int64_t>(),
                                                      degree.as<int>());
@@ -322,9 +290,9 @@ extern "C" int kb_umap_layout(kb_ctx* ctx, int64_t n, int64_t nnz, const int64_t
     UlStatus h;
     KB_CUDA(cudaMemcpyAsync(&h, d_st, sizeof(UlStatus), cudaMemcpyDeviceToHost, st));
     KB_CUDA(cudaStreamSynchronize(st));
-    if (h.flags & UL_BAD_INDPTR) { kb_set_error("umap layout: indptr must run from 0 to nnz and never decrease"); return KB_EINVAL; }
-    if (h.flags & UL_BAD_INDEX) { kb_set_error("umap layout: a column index is outside [0, n)"); return KB_EINVAL; }
-    if (h.flags & UL_BAD_DATA) { kb_set_error("umap layout: every weight must be finite and > 0"); return KB_EINVAL; }
+    if (h.flags & KB_CSR_BAD_INDPTR) { kb_set_error("umap layout: indptr must run from 0 to nnz and never decrease"); return KB_EINVAL; }
+    if (h.flags & KB_CSR_BAD_INDEX) { kb_set_error("umap layout: a column index is outside [0, n)"); return KB_EINVAL; }
+    if (h.flags & KB_CSR_BAD_DATA) { kb_set_error("umap layout: every weight must be finite and > 0"); return KB_EINVAL; }
     if (h.flags & UL_BAD_INIT) { kb_set_error("umap layout: the initial embedding holds a value that is not finite"); return KB_EINVAL; }
     const int64_t m = (int64_t)h.kept;
     *nnz_kept = m;

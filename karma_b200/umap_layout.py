@@ -91,17 +91,19 @@ def layout_graph(engine, graph, embedding, n_epochs, a, b, seed, gamma=1.0, init
     return out
 
 
-def _init_embedding(data, graph, n_components, init, random_state, metric, metric_kwds):
-    """umap 0.3.9's initial layout, drawing from ``random_state`` as umap does."""
+def _init_embedding(data, graph, n_components, init, random_state, metric, metric_kwds, spectral_layout=None):
+    """umap 0.3.9's initial layout, drawing from ``random_state`` as umap does.  ``spectral_layout``: the function
+    init="spectral" calls (default: ``umap.spectral.spectral_layout``)."""
     n = graph.shape[0]
     if isinstance(init, str) and init == "random":
         return random_state.uniform(low=-10.0, high=10.0, size=(n, n_components)).astype(np.float32)
     if isinstance(init, str) and init == "spectral":
-        try:
-            from umap.spectral import spectral_layout
-        except ImportError:
-            raise ValueError("init='spectral' needs umap-learn (umap.spectral.spectral_layout), which is not importable; "
-                             "pass init='random' or an array") from None
+        if spectral_layout is None:
+            try:
+                from umap.spectral import spectral_layout
+            except ImportError:
+                raise ValueError("init='spectral' needs umap-learn (umap.spectral.spectral_layout), which is not "
+                                 "importable; pass init='random', an array, or spectral_layout=") from None
         initialisation = spectral_layout(data, graph, n_components, random_state, metric=metric, metric_kwds=metric_kwds)
         expansion = 10.0 / np.abs(initialisation).max()
         return (initialisation * expansion).astype(np.float32) + random_state.normal(
@@ -121,12 +123,13 @@ def _init_embedding(data, graph, n_components, init, random_state, metric, metri
 
 
 def simplicial_set_embedding(data, graph, n_components, initial_alpha, a, b, gamma, negative_sample_rate, n_epochs, init,
-                             random_state, metric, metric_kwds, verbose=False, engine=None):
+                             random_state, metric, metric_kwds, verbose=False, engine=None, spectral_layout=None):
     """Drop-in for ``umap.umap_.simplicial_set_embedding`` of umap-learn 0.3.9: the same signature and host rules
     (n_epochs <= 0 -> 500 up to 10 000 rows, else 200; pruning; the initial layout from the pruned graph; ``rng_state``
     drawn last), the layout on
     the device.  Returns float32 [N, n_components].  ``random_state`` is a numpy RandomState, consumed exactly as umap
-    consumes it.  ``engine``: the GPU context (default: a new one)."""
+    consumes it.  ``engine``: the GPU context (default: a new one).  ``spectral_layout``: the function init="spectral"
+    calls instead of ``umap.spectral.spectral_layout``, with its signature (e.g. ``umap_spectral.spectral_layout``)."""
     import scipy.sparse
     if not (callable(metric) or metric in METRICS):
         raise ValueError("unknown metric %r" % (metric,))
@@ -141,7 +144,7 @@ def simplicial_set_embedding(data, graph, n_components, initial_alpha, a, b, gam
     # same max, which keeps every remaining edge.
     graph.data[graph.data < (graph.data.max() / float(n_epochs))] = 0.0
     graph.eliminate_zeros()
-    embedding = _init_embedding(data, graph, n_components, init, random_state, metric, metric_kwds)
+    embedding = _init_embedding(data, graph, n_components, init, random_state, metric, metric_kwds, spectral_layout)
     rng_state = random_state.randint(INT32_MIN, INT32_MAX, 3).astype(np.int64)
     csr = graph.tocsr()
     if engine is None:
