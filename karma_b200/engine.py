@@ -724,7 +724,7 @@ def _device_pass(engine, d_bases, d_offsets, d_key_len, n, kmer_size="5p6", n_ne
 
 def profile_and_knn(engine, bases, offsets, key_len, kmer_size="5p6", n_neighbors=None,
                     impl=KB_KNN_AUTO, want_profile=True, group=None, rank=0, world=1, row0=0, n_total=None,
-                    reuse_host=False, on_knn=None):
+                    reuse_host=False, on_knn=None, host_profile=True):
     """Run the hot path on host buffers (what KmerClustering and bench.py's e2e leg call).
 
     bases/offsets/key_len describe THIS rank's contigs (all of them when world==1).
@@ -738,6 +738,10 @@ def profile_and_knn(engine, bases, offsets, key_len, kmer_size="5p6", n_neighbor
     by the next call (a serving loop); otherwise every call returns fresh arrays.
     ``on_knn(idx, dist)`` is called as soon as the k-lists are on the host, before the profile download has
     finished (50k contigs, 5p6: about 4 ms against 8 ms for the whole call).
+
+    ``host_profile=False`` keeps the profile on the device for device consumers (``cluster.cluster_from_lists``):
+    the download is skipped, ``profile`` is None, and ``d_profile`` (float64 [n, D']) with ``d_idx`` (int32 [n, k])
+    and ``d_dist`` (float32 [n, k]) are device tensors.  The k-lists are still copied to ``knn_idx`` / ``knn_dist``.
     """
     n = len(offsets) - 1
     main = torch.cuda.current_stream(engine.device)
@@ -766,9 +770,11 @@ def profile_and_knn(engine, bases, offsets, key_len, kmer_size="5p6", n_neighbor
 
     r = device_pass(engine, d_bases, d_offsets, d_key_len, n, kmer_size, n_neighbors=n_neighbors, impl=impl,
                     want_profile=want_profile, group=group, rank=rank, world=world, n_total=n_total,
-                    on_profile=start_download if want_profile else None, row0=row0, chunks=chunks)
+                    on_profile=start_download if want_profile and host_profile else None, row0=row0, chunks=chunks)
     out = {"columns": r["columns"], "profile": None, "knn_idx": None, "knn_dist": None,
            "d_profile": r["profile"], "d_operand": r["operand"], "uncertified": r.get("uncertified", 0)}
+    if not host_profile:
+        out.update(d_idx=r["idx"], d_dist=r["dist"])
     if n_neighbors is not None:
         h_idx = engine.host_buffer("knn_idx", tuple(r["idx"].shape), torch.int32, reuse_host)
         h_dst = engine.host_buffer("knn_dist", tuple(r["dist"].shape), torch.float32, reuse_host)
@@ -780,7 +786,7 @@ def profile_and_knn(engine, bases, offsets, key_len, kmer_size="5p6", n_neighbor
         if on_knn is not None:
             # the k-lists are on the host now; the float64 profile (8*D' bytes per contig over PCIe) is still in flight
             on_knn(out["knn_idx"], out["knn_dist"])
-    if want_profile:
+    if want_profile and host_profile:
         side.synchronize()
         out["profile"] = hold["profile"].numpy()
     return out

@@ -17,6 +17,7 @@ karma.py keeps doing (karma.py:197-213)::
 import logging
 import os
 import sys
+import time
 
 import numpy as np
 
@@ -107,14 +108,22 @@ def umap_embedding(profile, knn_indices, knn_dists, umap_args, umap_module=None)
     return umap_module.UMAP(**umap_args).fit_transform(profile), "stock"
 
 
+CLUSTER_ROUTES = ("host", "device")
+
+
 class KmerClustering:
     """Mirror of kmer.py's class.  ``kmer_size``: "5p6" (kmer.py's default), an integer k (kmer.py:83-85): k <= 7
     counts into dense shared-memory histograms, 8 <= k <= 16 through sorted 128-bit k-mer keys, k > 16 raises
     KarmaB200Error (the sort key holds 16 characters); or the fixed-column throughput shapes "5+6" / "4+5" of this
     library (A/C/G/T only: other bytes are rejected there).  Sequences must be single-byte characters (latin-1;
-    FASTA is ASCII): one byte per character keeps byte order == the code-point order sorted() uses (kmer.py:172)."""
+    FASTA is ASCII): one byte per character keeps byte order == the code-point order sorted() uses (kmer.py:172).
 
-    def __init__(self, sequences, output_dir, kmer_size, threads):
+    ``cluster_on`` selects where UMAP and HDBSCAN run: "host" (umap-learn and hdbscan, through ``umap_embedding``)
+    or "device" (``cluster.cluster_from_lists``: the same stages as umap 0.3.9's route, on the GPU, with the profile
+    and the k-lists never downloaded for them).  None reads the environment variable KARMA_B200_CLUSTER, so that an
+    unmodified karma.py can choose; unset or empty means "host"."""
+
+    def __init__(self, sequences, output_dir, kmer_size, threads, cluster_on=None):
         # kmer.py:15-27
         self.sequences = sequences
         self.output_dir = output_dir
@@ -133,6 +142,13 @@ class KmerClustering:
         self.knn_indices = None
         self.knn_dists = None
         self._engine = None
+        self._d_knn = None
+
+        if cluster_on is None:
+            cluster_on = os.environ.get("KARMA_B200_CLUSTER") or "host"
+        if cluster_on not in CLUSTER_ROUTES:
+            raise ValueError("cluster_on (or KARMA_B200_CLUSTER) must be one of %s, got %r" % (CLUSTER_ROUTES, cluster_on))
+        self.cluster_on = cluster_on
 
     # ------------------------------------------------------------------ helpers
     @staticmethod
@@ -218,11 +234,13 @@ class KmerClustering:
             self._engine = Engine()
         return self._engine
 
-    def __calc_kmer_profile(self, n_neighbors=None):
+    def __calc_kmer_profile(self, n_neighbors=None, host_profile=True):
         """kmer.py:199-264 on the GPU.  Returns the float64 (N, D) profile; sets
         ``self.kmers`` ({kmer: column}) like the reference.  With ``n_neighbors``
         the exact kNN graph is computed in the same pass and left in
-        ``self.knn_indices`` / ``self.knn_dists``."""
+        ``self.knn_indices`` / ``self.knn_dists``.  With ``host_profile=False`` the
+        profile is returned as a device tensor and the device k-lists are left in
+        ``self._d_knn``."""
         from .engine import ZeroRowError, profile_and_knn
         logger.info("Extracting kmers from contigs.")               # kmer.py:152
         if self.kmer_size != "5p6":
@@ -233,7 +251,7 @@ class KmerClustering:
         bases, offsets, key_len = self._pack()
         try:
             res = profile_and_knn(self._get_engine(), bases, offsets, key_len, self.kmer_size,
-                                  n_neighbors=n_neighbors)
+                                  n_neighbors=n_neighbors, host_profile=host_profile)
         except ZeroRowError as e:
             # the column dictionary exists by the time the reference fails (kmer.py:202)
             logger.error(f"Values of row {e.row} are all zero, which should not be the case.")  # kmer.py:255-258
@@ -241,18 +259,48 @@ class KmerClustering:
         self.sorted_kmer_set = list(res["columns"])
         self.kmers = {kmer: i for i, kmer in enumerate(self.sorted_kmer_set)}   # kmer.py:175-177
         self.knn_indices, self.knn_dists = res["knn_idx"], res["knn_dist"]
-        kmer_profile = res["profile"]
+        kmer_profile = res["profile"] if host_profile else res["d_profile"]
+        if not host_profile:
+            self._d_knn = (res["d_idx"], res["d_dist"])
         self.sorted_kmer_set.clear()                                            # kmer.py:259
         logger.debug(f"KMER-PROFILE - Size: {sys.getsizeof(kmer_profile)}, Shape: {kmer_profile.shape}")
         return kmer_profile
 
+    def __cluster_on_device(self, neighbors, components, dist, r_state, min_cluster_size):
+        """The pass with the profile and k-lists kept on the device, then ``cluster_from_lists``.  Returns
+        (labels, probabilities); sets ``embedding`` (host float32), ``stage_ms`` and ``spectral_stats``."""
+        from .cluster import check_arguments, cluster_from_lists
+        k = check_arguments(len(self.sequences), neighbors, components, min_cluster_size)
+        logger.info("Calculate kmer profiles.")
+        t0 = time.perf_counter()
+        d_profile = self.__calc_kmer_profile(n_neighbors=k, host_profile=False)
+        pass_ms = (time.perf_counter() - t0) * 1e3
+        d_idx, d_dist = self._d_knn
+        self._d_knn = None
+        # UMAP and HDBSCAN are one device call here: both messages come before it
+        logger.info("Dimension reduction with UMAP.")
+        logger.info(f"Perform clustering with HDBSCAN. (min_cluster_size: {min_cluster_size})")
+        out = cluster_from_lists(self._get_engine(), d_idx, d_dist, d_profile, components, dist, r_state,
+                                 min_cluster_size)
+        self.umap_route = "device"
+        self.embedding = out["embedding"].cpu().numpy()
+        self.stage_ms = {"pass": pass_ms, **out["ms"]}
+        self.spectral_stats = out["spectral"]
+        return out["labels"], out["probabilities"]
+
     def run(self, neighbors, components, dist, r_state, min_cluster_size):
         """kmer.py:274-325: resume from cluster.txt if present, else profile (+ kNN) on the GPU,
-        UMAP, HDBSCAN, write cluster.txt / eval.txt."""
+        UMAP, HDBSCAN, write cluster.txt / eval.txt.  UMAP and HDBSCAN run where ``cluster_on`` says."""
         if os.path.isfile(self.output_file):
             logger.info(f"Read from previous calculation: {self.output_file}")
             self.__read_clusters()
             self.__fix_fasta_headers()
+            return
+        if self.cluster_on == "device":
+            labels, probabilities = self.__cluster_on_device(neighbors, components, dist, r_state, min_cluster_size)
+            t0 = time.perf_counter()
+            self.__write_results(labels, probabilities, neighbors, components, dist, r_state, min_cluster_size)
+            self.stage_ms["files"] = (time.perf_counter() - t0) * 1e3
             return
 
         logger.info("Calculate kmer profiles.")
@@ -272,13 +320,16 @@ class KmerClustering:
         import hdbscan
         hdb_args = {"allow_single_cluster": True} if min_cluster_size == 1 else {"min_cluster_size": min_cluster_size}
         clusterer = hdbscan.HDBSCAN(**hdb_args).fit(embedding)
-        labels = clusterer.labels_
+        self.__write_results(clusterer.labels_, clusterer.probabilities_, neighbors, components, dist, r_state,
+                             min_cluster_size)
 
+    def __write_results(self, labels, probabilities, neighbors, components, dist, r_state, min_cluster_size):
+        """The end of kmer.py's run: groups, cluster.txt, eval.txt, then the header fix."""
         self.clusters, self.unlabeled_cluster = self.__mask_list(self.sequences, labels)
         self.__save_groups_to_file()
         self.__write_eval_information(
             kmer_size=self.kmer_size, n_neighbors=neighbors, n_components=components, min_dist=dist,
             random_state=r_state, min_cluster_size=min_cluster_size,
             unlabeled=list(labels).count(-1), no_groups=max(labels) + 1,
-            mean_probability=np.mean(clusterer.probabilities_))
+            mean_probability=np.mean(probabilities))
         self.__fix_fasta_headers()

@@ -135,10 +135,11 @@ def _layout(engine, res, random_state):
     return assemble(engine, res, u)
 
 
-def spectral_init(engine, graph, dim, n_epochs, random_state, data=None):
+def spectral_init(engine, graph, dim, n_epochs, random_state, data=None, return_build=False):
     """K7's device graph in, the device float32 [N, dim] initial layout for ``layout_graph`` out: umap 0.3.9's
     spectral_layout on the graph pruned at max / n_epochs, then ``_init_embedding``'s expansion to 10 / max|.| and its
-    ``normal(scale=1e-4)`` noise.  ``random_state`` (a numpy RandomState) is consumed exactly as umap consumes it."""
+    ``normal(scale=1e-4)`` noise.  ``random_state`` (a numpy RandomState) is consumed exactly as umap consumes it.
+    With ``return_build`` also ``spectral_build``'s dict (components, status, Lanczos statistics)."""
     if not isinstance(random_state, np.random.RandomState):
         raise ValueError("random_state must be a numpy RandomState")
     res = spectral_build(engine, graph, dim, n_epochs, data)
@@ -151,7 +152,8 @@ def spectral_init(engine, graph, dim, n_epochs, random_state, data=None):
         expansion = np.float32(10.0) / np.float32(init.abs().max().item())
         init = init * torch.tensor(expansion, dtype=torch.float32, device=engine.device)
     noise = random_state.normal(scale=0.0001, size=[n, dim]).astype(np.float32)
-    return init + torch.from_numpy(noise).to(engine.device)
+    init = init + torch.from_numpy(noise).to(engine.device)
+    return (init, res) if return_build else init
 
 
 def spectral_layout(data, graph, dim, random_state, metric="euclidean", metric_kwds={}, engine=None):
