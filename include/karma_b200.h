@@ -485,6 +485,35 @@ KB_API int kb_spectral_fetch(kb_ctx* ctx, int32_t* h_size, int32_t* h_status, do
                    int32_t* d_labels, double* d_meta, double* d_vectors, double* d_centroids);
 KB_API int kb_spectral_assemble(kb_ctx* ctx, const double* d_u, float* d_out);
 
+/* ---- K11: MCL of many groups of a read graph in one call ----
+ * Replaces karma's `mcl - --abc -o -` per k-mer cluster (Mcl.run_pipe); the semantics are this library's definition,
+ * frozen in oracle/mcl_oracle.py (DESIGN §3 K11 lists the parts that rest on memory of mcl 14-137, unpinned).
+ * Group g's abc stream is the edges with both ends in g, in edge order; its nodes are numbered by first appearance
+ * (a before b).  A = adjacency + loops A[j,j] = max_i A[i,j]; M = A / column sums; until g's chaos
+ * max_j (max_i M[i,j] / sum_i M[i,j]^2 - 1) < 1e-4, each iteration expands (M*M, terms in ascending k), prunes every
+ * column (cutoff 1/7000, the 900 largest, recovery up to 1000 entries or 90 % of the mass; ties by row), inflates
+ * (x^inflation) and renormalises.  fp64, no FMA, every sum a left fold in ascending rows: the same inputs give the same
+ * bits.  Every group iterates until its own convergence, so its result does not depend on the other groups.
+ * Interpretation: attractors M[a,a] > 0, systems = connected attractors numbered by their smallest attractor, each node
+ * to the smallest system it reaches (alone if none); clusters ordered by size desc, then smallest member.
+ * kb_mcl_build (device pointers; synchronises once per iteration; keeps the result on the host side of the context):
+ *  d_a, d_b int32[n_edges]  edge ends in [0, n_nodes); d_w double[n_edges]
+ *  d_group  int32[n_nodes]  group ids in [-1, n_groups), -1 = in no group
+ *  inflation finite and > 1
+ *  KB_EINVAL for an index or group id out of range, and inside a group for a self-edge, a pair listed twice or a weight
+ *  that is not finite and > 0; also for a group that has not converged after 1000 iterations (the message names it).
+ *  n_cols out: the nodes in streams; nnz out: the entries of the final matrix.
+ * kb_mcl_fetch (host pointers, any may be NULL): h_local int32[n_nodes] (stream index, -1 outside every stream),
+ *  h_cluster int32[n_nodes] (cluster number within the group, in output order; -1 outside), h_n_clusters,
+ *  h_iterations, h_overlap int64[n_groups] (overlap: nodes reaching attractors of several systems), and the final
+ *  matrix: h_colptr int64[n_cols + 1] (columns group by group, stream index within), h_rows int32[nnz] (stream
+ *  indices, ascending per column), h_vals double[nnz]. */
+KB_API int kb_mcl_build(kb_ctx* ctx, int64_t n_nodes, int64_t n_edges, const int32_t* d_a, const int32_t* d_b,
+                   const double* d_w, const int32_t* d_group, int64_t n_groups, double inflation, int64_t* n_cols,
+                   int64_t* nnz);
+KB_API int kb_mcl_fetch(kb_ctx* ctx, int32_t* h_local, int32_t* h_cluster, int64_t* h_n_clusters, int64_t* h_iterations,
+                   int64_t* h_overlap, int64_t* h_colptr, int32_t* h_rows, double* h_vals);
+
 /* Per-stage device times.  With timing enabled every launch of a stage is bracketed
  * by a CUDA-event pair on the context stream (a ring of 128 pairs per stage).
  * kb_stage_ms synchronises, returns the mean duration (ms) and the number of launches
@@ -493,7 +522,8 @@ KB_API int kb_spectral_assemble(kb_ctx* ctx, const double* d_u, float* d_out);
  *         7 read-graph build, 8 group-pair connection weights, 9 K9 core distances, 10 K9 Boruvka rounds (one launch
  *         recorded per round), 11 K9 edge sort, 12 K10 components (validation, pruning, component rounds, labels and
  *         the permuted CSR), 13 K10 eigensolve (every component solve, host Ritz steps included), 14 K10 meta-embedding
- *         (centroids, affinity, the meta solve, data ranges) */
+ *         (centroids, affinity, the meta solve, data ranges), 15 K11 set-up (validation, labelling, the initial matrix),
+ *         16 K11 iteration (one launch recorded per iteration) */
 KB_API int kb_enable_timing(kb_ctx* ctx, int on);
 KB_API int kb_stage_ms(kb_ctx* ctx, int which, float* mean_ms, int* n_launches);
 /* Number of kernels this library launched since the context was created (a CUB device-wide call counts as one). */

@@ -19,7 +19,7 @@ KB_COUNT_NO_COLUMNS = 0x100
 
 STAGES = {"count": 0, "count_long": 1, "compact": 2, "normalise": 3, "knn_gemm": 4, "rerank": 5, "knn_exact": 6, "readgraph": 7, "links": 8,
           "hdbscan_core": 9, "hdbscan_mst": 10, "hdbscan_sort": 11, "spectral_components": 12, "spectral_eigensolve": 13,
-          "spectral_meta": 14}
+          "spectral_meta": 14, "mcl_setup": 15, "mcl_iteration": 16}
 
 
 def KB_MODE_K(k):
@@ -88,6 +88,8 @@ SIGNATURES = {
     "kb_spectral_build": (c_int, [_P, c_int64, c_int64, _P, _P, _P, c_int32, c_int32, _P, c_int32, c_int64, POINTER(c_int64)]),
     "kb_spectral_fetch": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "kb_spectral_assemble": (c_int, [_P, _P, _P]),
+    "kb_mcl_build": (c_int, [_P, c_int64, c_int64, _P, _P, _P, _P, c_int64, c_double, POINTER(c_int64), POINTER(c_int64)]),
+    "kb_mcl_fetch": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "kb_enable_timing": (c_int, [_P, c_int]),
     "kb_stage_ms": (c_int, [_P, c_int, POINTER(c_float), POINTER(c_int)]),
     "kb_launch_count": (c_int64, [_P]),

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "libkarma_b200.so")
-SOURCES = ["kb_api.cu", "kb_count.cu", "kb_profile.cu", "kb_exotic.cu", "kb_knn.cu", "kb_knn_tc.cu", "kb_xchg.cu", "kb_fasta.cu", "kb_readgraph.cu", "kb_links.cu", "kb_umapgraph.cu", "kb_umaplayout.cu", "kb_hdbscan.cu", "kb_spectral.cu"]
+SOURCES = ["kb_api.cu", "kb_count.cu", "kb_profile.cu", "kb_exotic.cu", "kb_knn.cu", "kb_knn_tc.cu", "kb_xchg.cu", "kb_fasta.cu", "kb_readgraph.cu", "kb_links.cu", "kb_umapgraph.cu", "kb_umaplayout.cu", "kb_hdbscan.cu", "kb_spectral.cu", "kb_mcl.cu"]
 HEADERS = ["kb_common.cuh", "kb_knn.cuh", os.path.join("..", "..", "include", "karma_b200.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]

@@ -35,7 +35,7 @@ int kb_mode_describe(int mode, KbMode* m) {
     return KB_OK;
 }
 
-extern "C" int kb_version(void) { return 104; }
+extern "C" int kb_version(void) { return 105; }
 extern "C" const char* kb_last_error(void) { return g_err; }
 
 extern "C" int kb_mode_columns(int mode) {
@@ -91,6 +91,7 @@ extern "C" int kb_destroy(kb_ctx* c) {
     kb_fuzzy_free(c);
     kb_knn_cache_free(c);
     kb_spectral_free(c);
+    kb_mcl_free(c);
     if (c->pool) { cudaDeviceSynchronize(); cudaMemPoolDestroy(c->pool); }
     free(c);
     return KB_OK;

@@ -8,7 +8,7 @@
 #include <nvtx3/nvToolsExt.h>          // header-only (NVTX v3): ranges are no-ops unless a profiler is attached
 #include "../../include/karma_b200.h"
 
-#define KB_N_TIMERS 15
+#define KB_N_TIMERS 17
 #define KB_EV_RING 128
 
 struct kb_ctx {
@@ -45,6 +45,8 @@ struct kb_ctx {
     void* knn_cache;
     // the spectral initialisation of the last kb_spectral_build (kb_spectral.cu, owned)
     void* spectral;
+    // the MCL result of the last kb_mcl_build (kb_mcl.cu, owned)
+    void* mcl;
 };
 
 void kb_set_error(const char* fmt, ...);
@@ -67,7 +69,7 @@ static const char* const kb_stage_names[KB_N_TIMERS] = {
     "kb:K1 count", "kb:K1 count (split contigs)", "kb:K2 compact", "kb:K3 normalise", "kb:K4 distance GEMM + top-k",
     "kb:K5 merge + exact rerank", "kb:K4x/K6 exact distances", "kb:read graph", "kb:group links",
     "kb:K9 core distances", "kb:K9 Boruvka round", "kb:K9 edge sort", "kb:K10 components", "kb:K10 eigensolve",
-    "kb:K10 meta-embedding"};
+    "kb:K10 meta-embedding", "kb:K11 set-up", "kb:K11 iteration"};
 struct KbTimer {
     kb_ctx* c; int which; int slot;
     KbTimer(kb_ctx* ctx, int w) : c(ctx), which(w), slot(0) {
@@ -101,6 +103,7 @@ void kb_links_free(kb_ctx* c);
 void kb_fuzzy_free(kb_ctx* c);
 void kb_knn_cache_free(kb_ctx* c);
 void kb_spectral_free(kb_ctx* c);
+void kb_mcl_free(kb_ctx* c);
 // host-side file input shared by the FASTA and eq_classes parsers (kb_fasta.cu)
 int64_t kb_host_threads();
 int kb_host_read_file(const char* path, uint8_t** img, int64_t* size);
